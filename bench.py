@@ -2,6 +2,7 @@
 """bench.py — simulated Gbp/s of the PBSIM3 read-generation hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c1|c2|c4|c5|cs] [--impl reference]
+                    [--dump-outputs DIR]
 
 A STEP is one call of the reference's seam for one reference sequence: ingest the sequence
 (get_genome_seq), then simulate_by_qshmm / simulate_by_errhmm to the depth quota, records emitted
@@ -552,7 +553,7 @@ def measure(W, my_parts, warm_parts, e2e_steps, barrier, dist=None, read_range=N
     for lane in range(dev_lanes):
         W.engine(lane).timer_start()
     t0 = time.perf_counter()
-    acc = dict(bases=0, out_bytes=0, launches=0, sim=0.0, emit=0.0, seg=0.0, chain=0.0, gen=0.0)
+    acc = dict(bases=0, out_bytes=0, launches=0, sim=0.0, emit=0.0, seg=0.0, chain=0.0, gen=0.0, done=[])
 
     tp = [time.perf_counter()]
 
@@ -571,6 +572,7 @@ def measure(W, my_parts, warm_parts, e2e_steps, barrier, dist=None, read_range=N
         acc["seg"] += st.seg_seconds
         acc["chain"] += st.chain_seconds
         acc["gen"] += st.gen_seconds
+        acc["done"].append((p, st))
 
     run_parts(W, my_parts, dist, True, on_part, read_range=read_range, lanes=dev_lanes)
     # CUDA events on every engine's own stream, all started behind the same device-wide synchronisation: the span of
@@ -630,8 +632,8 @@ def measure(W, my_parts, warm_parts, e2e_steps, barrier, dist=None, read_range=N
 
             run_parts(W, parts_e, dist, False, on_e, read_range=read_range, host_seq=host_seq, sink=sink, lanes=e2e_lanes)
             barrier()
-            return dict(e, ms=(time.perf_counter() - t0) * 1e3, steps=len(set(p["seq"] for p in parts_e)) if W.seqset is None
-                        else len(parts_e))
+            # a step is one run of a sequence (or of the set): exactly one of its parts is the last one
+            return dict(e, ms=(time.perf_counter() - t0) * 1e3, steps=sum(1 for p in parts_e if p["last"]))
 
         # untimed: one run through every engine of the arm, so that pinned staging buffers and record buffers exist
         if parts_e:
@@ -746,6 +748,100 @@ def verify_split(W, my_parts, dist, rank):
     return out
 
 
+# --dump-outputs: per record stream (FASTQ or SAM, MAF) its first DUMP_HEAD bytes and DUMP_SAMPLE bytes at seeded
+# positions over the whole stream (a c3 step writes tens of GB); with the statistics the files take 32 MiB
+DUMP_HEAD = 2 << 20
+DUMP_SAMPLE = 2 << 20
+DUMP_SEED = 20240502
+DUMP_STATS = ("res_num", "res_pass_num", "res_len_total", "res_len_min", "res_len_max", "res_sub_num", "res_ins_num",
+              "res_del_num", "accuracy_total", "res_len_mean", "res_len_sd", "res_accuracy_mean", "res_accuracy_sd",
+              "len_total_end")
+
+
+class _HbmBytes:
+    """n bytes of device memory at ptr, for torch.as_tensor (CUDA array interface, no copy)"""
+
+    def __init__(self, ptr, n):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "|u1", "data": (ptr, False), "strides": None,
+                                         "version": 2}
+
+
+class StreamSample:
+    """the first `head` bytes of a byte stream that arrives in pieces, and its bytes at the sorted positions `pos`"""
+
+    def __init__(self, pos, head):
+        self.pos, self.head_n, self.off, self.head, self.sample = pos, head, 0, [], []
+
+    def feed(self, t):
+        """t: the next piece, a 1-D uint8 tensor on any device"""
+        import numpy as np
+        import torch
+        n = t.numel()
+        if self.off < self.head_n:
+            self.head.append(t[:self.head_n - self.off].cpu())
+        lo, hi = np.searchsorted(self.pos, [self.off, self.off + n])
+        if hi > lo:
+            self.sample.append(t[torch.from_numpy(self.pos[lo:hi] - self.off).to(t.device)].cpu())
+        self.off += n
+
+    def arrays(self):
+        """(head, sample), one float32 per byte"""
+        import numpy as np
+        import torch
+        return [(torch.cat(x).numpy() if x else np.zeros(0, np.uint8)).astype(np.float32) for x in (self.head, self.sample)]
+
+
+def dump_outputs(W, parts, done, read_range, out_dir):
+    """What the last timed step computed, as .npy files in out_dir: for reads (FASTQ or SAM records) and maf,
+    <stream>_head.npy (the first DUMP_HEAD bytes) and <stream>_sample.npy (the bytes at DUMP_SAMPLE positions drawn
+    with DUMP_SEED over the stream's length), each byte as a float32; stats.npy (float64) = DUMP_STATS, emitted bases,
+    reads bytes, maf bytes.  Every batch of the device arm overwrites the records of the previous one, so the step
+    runs again, untimed, on the same engine: once to learn the streams' lengths, once to copy the bytes out.  A read
+    depends only on seed, sequence and read number; both runs must end with the timed step's statistics.
+    Returns what the JSON line reports: the directory, the step's sequence (a sequence set counts as sequence 1), its
+    length and the number of batches its records came in."""
+    import numpy as np
+    import torch
+    from pbsim_b200 import stats_reduce as SR
+    order = [p for phase in SR.split_order(parts) for p in phase]
+    last = order[-1]
+    want = [float(getattr(st, f)) for p, st in done if p is last for f in DUMP_STATS]
+
+    def rerun(on_chunk):
+        # rng_seed: run_parts seeds the runs of a sequence set by their place in the order
+        b, _, st = W.run_part(last, rng_seed=len(order) - 1, read_range=read_range, on_chunk=on_chunk)
+        got = [float(getattr(st, f)) for f in DUMP_STATS]
+        if got != want:
+            raise RuntimeError("--dump-outputs: the untimed run of the last step differs from the timed one: %s != %s"
+                               % (dict(zip(DUMP_STATS, got)), dict(zip(DUMP_STATS, want))))
+        return b
+
+    totals = [0, 0, 0]  # reads bytes, maf bytes, batches
+
+    def count(c):
+        totals[0] += c.reads_bytes
+        totals[1] += c.maf_bytes
+        totals[2] += 1
+
+    rerun(count)
+    rng = np.random.default_rng(DUMP_SEED)
+    streams = [StreamSample(np.unique(rng.integers(0, max(1, n), DUMP_SAMPLE)), DUMP_HEAD) for n in totals[:2]]
+
+    def gather(c):
+        torch.cuda.synchronize()  # the engine's kernels run on its own streams
+        for s, ptr, n in zip(streams, (c.reads, c.maf), (c.reads_bytes, c.maf_bytes)):
+            if n:
+                s.feed(torch.as_tensor(_HbmBytes(ptr, n)))
+
+    bases = rerun(gather)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, s in zip(("reads", "maf"), streams):
+        for kind, a in zip(("head", "sample"), s.arrays()):
+            np.save(os.path.join(out_dir, "%s_%s.npy" % (name, kind)), a)
+    np.save(os.path.join(out_dir, "stats.npy"), np.array(want + [bases] + totals[:2], dtype=np.float64))
+    return {"dir": out_dir, "sequence": last["seq"] + 1, "sequence_bp": W.contigs[last["seq"]], "batches": totals[2]}
+
+
 def roofline_block(method, acc, peak, peak_src):
     """whole-step fraction on top; per-kernel fractions (each kernel against its OWN algorithmic bytes) below"""
     bases = acc["bases"]
@@ -818,7 +914,13 @@ def main():
     ap.add_argument("--verify-split", action="store_true",
                     help="N > 1: after the timed runs, rank 0 simulates every shared sequence whole and compares the "
                          "CRC-32 of its bytes, cut at the parts' byte counts, with what the ranks delivered")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU: after the timed steps, write what the last of them computed to DIR as .npy files "
+                         "(a seeded sample of its records and its statistics, see dump_outputs), so that two builds "
+                         "can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        raise SystemExit("--dump-outputs needs --impl ours and at least one timed step")
     if args.impl == "reference":
         reference_arm(args, dict(WORKLOADS[args.workload]))
         return
@@ -830,6 +932,8 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the engine has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs runs on one GPU")
     torch.cuda.set_device(local)
     pin_to_gpu_numa_node(local)
     dist = None
@@ -923,6 +1027,7 @@ def main():
     acc = measure(W, mine, warm, args.e2e_steps, barrier, dist=dist, read_range=read_range, e2e_lanes=args.e2e_lanes,
                   parts_e=parts_e, dev_lanes=args.lanes)
     clocks = sampler.stop()
+    dumped = dump_outputs(W, mine, acc["done"], read_range, args.dump_outputs) if args.dump_outputs else None
 
     verified = None
     if args.verify_split and dist is not None and split_info is not None:
@@ -967,6 +1072,8 @@ def main():
         }
         if per_rank is not None:
             line["per_rank"] = per_rank
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         if split_info is not None:
             line["split"] = split_info
             if verified is not None:
