@@ -45,28 +45,27 @@ namespace {
 
 thread_local std::string g_create_error;
 
+// Device memory that grows on demand and is freed with its owner (the engine is deleted on the engine's device).
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
-  cudaError_t ensure(size_t bytes, bool keep = false, cudaStream_t st = 0) {
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  ~DevBuf() { cudaFree(p); }  // no-op for nullptr
+  cudaError_t ensure(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     size_t want = bytes + bytes / 8 + 256;
     void *np = nullptr;
     cudaError_t e = cudaMalloc(&np, want);
     if (e != cudaSuccess) return e;
     if (p) {
-      if (keep) cudaMemcpyAsync(np, p, cap, cudaMemcpyDeviceToDevice, st);
-      cudaStreamSynchronize(st);
+      cudaStreamSynchronize(0);
       cudaFree(p);
     }
     p = np;
     cap = want;
     return cudaSuccess;
-  }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
   }
   template <class T>
   T *as() const { return reinterpret_cast<T *>(p); }
@@ -75,6 +74,10 @@ struct DevBuf {
 struct PinnedBuf {
   void *p = nullptr;
   size_t cap = 0;
+  PinnedBuf() = default;
+  PinnedBuf(const PinnedBuf &) = delete;
+  PinnedBuf &operator=(const PinnedBuf &) = delete;
+  ~PinnedBuf() { release(); }
   cudaError_t ensure(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) cudaFreeHost(p);
@@ -236,13 +239,13 @@ struct pbsim_engine {
   // batch arrays
   DevBuf b_read_u32;   // 5 arrays per read (carve_batch)
   DevBuf b_sub_u32;    // 16 arrays per subread
-  DevBuf b_sub_u64;    // 12 slices of n_sub + 1 (u64_slice)
+  DevBuf b_sub_u64;    // kU64Slices slices of n_sub + 1 (u64_slice)
   DevBuf b_sub_f64;
-  DevBuf d_bins;       // bin_start[kBins+1], bin_lo[kBins], bin_hi[kBins], cta_first[kBins+1]
+  DevBuf d_bins;       // pass-1 CTA schedule of the sub-reads (schedule_ctas)
   DevBuf d_ctrl;       // control words
   DevBuf d_cub_tmp;
   DevBuf d_ev, d_ck, d_lay, d_tile_sub, d_tile_desc;
-  DevBuf d_seg, d_seg_bins;       // segment-parallel pass 1: segment lists / results, CTA map
+  DevBuf d_seg, d_seg_bins;       // segment-parallel pass 1: segment lists / results, CTA schedule
   int seg_enabled = 1;            // option "segments"
   int64_t seg_min_len = 2048;     // option "seg_min_len": shorter reads stay on the sequential path
   int64_t seg_batches = 0, seg_fallback_batches = 0;
@@ -446,6 +449,15 @@ int upload_bias_tables(pbsim_engine *e) {
   return 0;
 }
 
+// the sequence text into d_ascii, zero-padded to a multiple of 16 and 64 bytes more; bases == nullptr: a kernel writes it
+int upload_ascii(pbsim_engine *e, const char *bases, int64_t len) {
+  const size_t padded = ((size_t)len + 15) / 16 * 16 + 64;
+  CK(e->d_ascii.ensure(padded));
+  CK(cudaMemsetAsync(e->d_ascii.as<uint8_t>() + (len / 16) * 16, 0, padded - (len / 16) * 16, e->st));
+  if (bases) CK(cudaMemcpyAsync(e->d_ascii.p, bases, (size_t)len, cudaMemcpyHostToDevice, e->st));
+  return 0;
+}
+
 // keep_first: sequence sets whose first base keeps its case (see k_set_restore_first)
 int finish_sequence_ingest(pbsim_engine *e, int64_t len, int32_t seq_num, const double bias[12], bool keep_first = false) {
   // ascii already in d_ascii (padded with zeros to a multiple of 16)
@@ -519,13 +531,21 @@ struct BatchResult {
   uint64_t bases_all = 0;
 };
 
+// slices of b_sub_u64, each n_sub + 1 long; kSliceScanIn is the input of a scan (widened counts, pass-0 lengths)
+enum U64Slice { kSliceEvOff, kSliceCkOff, kSliceScanIn, kSliceRlen0Prefix, kSliceReadsSize, kSliceMafSize, kSliceNtiles,
+                kSliceReadsOff, kSliceMafOff, kSliceTileStart, kSliceSegOff, kSliceChunkOff, kU64Slices };
+
+inline unsigned long long *u64_slice(pbsim_engine *e, U64Slice k) {
+  return e->b_sub_u64.as<unsigned long long>() + (size_t)k * (e->B.n_sub + 1);
+}
+
 int carve_batch(pbsim_engine *e, uint32_t n_reads) {
   const uint32_t pass = (uint32_t)e->model.pass_num;
   const uint64_t n_sub = (uint64_t)n_reads * pass;
   if (n_sub > 0x7FFFFFFFull) return fail(e, PBSIM_E_INVALID, "batch too large");
   CK(e->b_read_u32.ensure((size_t)n_reads * 7 * 4 + 64));
   CK(e->b_sub_u32.ensure((size_t)n_sub * 16 * 4 + 64));
-  CK(e->b_sub_u64.ensure((size_t)(n_sub + 1) * 12 * 8 + 64));
+  CK(e->b_sub_u64.ensure((size_t)(n_sub + 1) * kU64Slices * 8 + 64));
   CK(e->b_sub_f64.ensure((size_t)n_sub * 8 + 64));
   Batch &B = e->B;
   B.n_reads = n_reads;
@@ -542,16 +562,11 @@ int carve_batch(pbsim_engine *e, uint32_t n_reads) {
   uint32_t **fields[] = {&B.key_in, &B.key_out, &B.idx_in, &B.order, &B.cap, &B.ck_cap, &B.nent, &B.rlen,
                          &B.ncol, &B.nsub, &B.nins, &B.ndel, &B.flags, &B.draws_used, &B.nseg, &B.nchunk};
   for (size_t i = 0; i < sizeof(fields) / sizeof(fields[0]); ++i) *fields[i] = s32 + i * n_sub;
-  uint64_t *s64 = e->b_sub_u64.as<uint64_t>();
-  B.ev_off = s64;
-  B.ck_off = s64 + (n_sub + 1);
+  B.ev_off = reinterpret_cast<uint64_t *>(u64_slice(e, kSliceEvOff));
+  B.ck_off = reinterpret_cast<uint64_t *>(u64_slice(e, kSliceCkOff));
   B.accuracy = e->b_sub_f64.as<double>();
   return 0;
 }
-
-// slices of b_sub_u64 (each n_sub + 1 long): 0 ev_off, 1 ck_off, 2 tmp widen, 3 rlen0 prefix,
-// 4 reads_size, 5 maf_size, 6 ntiles, 7 reads_off, 8 maf_off, 9 tile_start, 10 seg_off, 11 chunk_off
-inline uint64_t *u64_slice(pbsim_engine *e, int k) { return e->b_sub_u64.as<uint64_t>() + (size_t)k * (e->B.n_sub + 1); }
 
 int excl_scan(pbsim_engine *e, const unsigned long long *in, unsigned long long *out, uint32_t n) {
   size_t tmp = 0;
@@ -562,403 +577,332 @@ int excl_scan(pbsim_engine *e, const unsigned long long *in, unsigned long long 
   return 0;
 }
 
-// sb: --method sample, the groups of this batch (n_reads = their copies); otherwise null
-int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult *out, const SampleBatch *sb = nullptr) {
-  const uint32_t pass = (uint32_t)e->model.pass_num;
-  const bool qs = e->model.method != PBSIM_METHOD_ERRHMM;  // sample reads use the qshmm event stream
-  const bool sample = e->model.method == PBSIM_METHOD_SAMPLE;
-  DevicePool Pl;
-  Pl.quals = e->d_pool_q.as<uint8_t>();
-  Pl.start = e->d_pool_start.as<uint64_t>();
-  Pl.n = (uint32_t)(e->pool_start.empty() ? 0 : e->pool_start.size() - 1);
-  if (sample && !sb) return fail(e, PBSIM_E_INVALID, "internal: sample batch without groups");
-  const bool spec = sample && e->sample_spec && e->sample_spec_run;
-  const bool replay = e->run.rng_mode == PBSIM_RNG_REPLAY;
-  int rc = carve_batch(e, n_reads);
+// out[0..n] = exclusive sum of the uint32 in[0..n), out[n] the total.  tmp holds n + 1 words; the scan reads tmp[n],
+// which k_widen does not write and which does not change the sum
+int widen_scan(pbsim_engine *e, const uint32_t *in, uint32_t n, unsigned long long *tmp, unsigned long long *out) {
+  k_widen<<<nblk(n, 256), 256, 0, e->st>>>(in, n, tmp);
+  e->launches++;
+  return excl_scan(e, tmp, out, n + 1);
+}
+
+int sort_pairs(pbsim_engine *e, const uint32_t *keys_in, uint32_t *keys_out, const uint32_t *vals_in, uint32_t *vals_out,
+               uint32_t n, int begin_bit, int end_bit) {
+  size_t tmp = 0;
+  CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, keys_in, keys_out, vals_in, vals_out, (int)n, begin_bit, end_bit, e->st));
+  CK(e->d_cub_tmp.ensure(tmp + 256));
+  tmp = e->d_cub_tmp.cap;
+  CK(cub::DeviceRadixSort::SortPairs(e->d_cub_tmp.p, tmp, keys_in, keys_out, vals_in, vals_out, (int)n, begin_bit, end_bit,
+                                     e->st));
+  return 0;
+}
+
+// the CTAs of one pass: bin b (accuracy * 2 + slow, sim_kernels.cuh) holds the sorted items
+// [bin_lo[b], bin_hi[b]) and owns the CTAs from cta_first[b]; CTA slot i runs CTA order[i]
+struct CtaSchedule {
+  uint32_t *bin_start, *bin_lo, *bin_hi, *cta_first, *order;
+  uint32_t slots;
+};
+
+// Sorts the items by key bits [begin_bit, 28) (ids_out: the items in that order), bins them and maps the bins to CTAs
+// of cta_threads items.  longest_first orders the CTAs by their first key (k_cta_keys), otherwise they run in bin
+// order.  The arrays are carved from buf.  Counts its 4 launches; CUB's are not counted.
+int schedule_ctas(pbsim_engine *e, DevBuf &buf, const uint32_t *keys_in, uint32_t *keys_out, const uint32_t *ids_in,
+                  uint32_t *ids_out, uint32_t n, int begin_bit, uint32_t cta_threads, bool longest_first,
+                  CtaSchedule *s) {
+  s->slots = nblk(n, cta_threads) + kBins;
+  CK(buf.ensure((4 * kBins + 8) * 4 + (size_t)s->slots * 4 * 4 + 64));
+  s->bin_start = buf.as<uint32_t>();
+  s->bin_lo = s->bin_start + kBins + 1;
+  s->bin_hi = s->bin_lo + kBins;
+  s->cta_first = s->bin_hi + kBins;
+  uint32_t *cta_key = s->cta_first + kBins + 1, *cta_id = cta_key + s->slots, *cta_key_s = cta_id + s->slots;
+  s->order = cta_key_s + s->slots;
+  int rc = sort_pairs(e, keys_in, keys_out, ids_in, ids_out, n, begin_bit, 28);
   if (rc) return rc;
+  k_fill_u32<<<1, 256, 0, e->st>>>(s->bin_start, kBins + 1, 0xFFFFFFFFu);
+  k_bin_bounds<<<nblk(n, 256), 256, 0, e->st>>>(keys_out, n, s->bin_start);
+  k_cta_map<<<1, 32, 0, e->st>>>(s->bin_start, keys_out, n, s->bin_lo, s->bin_hi, s->cta_first, cta_threads);
+  e->launches += 4;
+  if (!longest_first) {
+    k_iota_u32<<<nblk(s->slots, 256), 256, 0, e->st>>>(s->order, s->slots);
+    return 0;
+  }
+  k_cta_keys<<<nblk(s->slots, 256), 256, 0, e->st>>>(keys_out, s->bin_lo, s->cta_first, s->slots, cta_key, cta_id,
+                                                    cta_threads);
+  return sort_pairs(e, cta_key, cta_key_s, cta_id, s->order, s->slots, 0, 21);
+}
+
+// the CTA map of a schedule in kernel arguments (SimArgs, SegArgs)
+template <class Args>
+void set_ctas(Args &a, const CtaSchedule &s) {
+  a.cta_order = s.order;
+  a.cta_first = s.cta_first;
+  a.bin_lo = s.bin_lo;
+  a.bin_hi = s.bin_hi;
+}
+
+// what the phases of one batch share besides the engine and its batch arrays (e->B)
+struct BatchCtx {
+  uint32_t pass, cta_threads;
+  int64_t clip_room;       // >= 0: the one read of a tail batch is clipped to this many bases
+  const SampleBatch *sb;   // --method sample: the groups of this batch (n_reads = their copies); otherwise null
+  bool qs, sample, spec, replay;
+  DevicePool Pl;
+  SimArgs A;                 // pass-1 arguments; their model M, genome G and generator rng serve every phase
+  int64_t next_start_after = -1;  // replay: draw-log start of the subread behind the batch (-1: none)
+  // the current attempt
+  bool use_segments;
+  CtaSchedule cta;  // pass-1 CTAs of the sub-reads
+  uint64_t n_seg_total, n_chunk_total;
+};
+
+inline unsigned long long *host_ctrl(pbsim_engine *e) { return reinterpret_cast<unsigned long long *>(e->h_ctrl.p); }
+
+// replay: upload the slice of the draw log this batch can touch
+int upload_replay_window(pbsim_engine *e, BatchCtx &c) {
+  const int64_t s0 = (int64_t)(e->next_read - e->run.first_read) * c.pass, n_sub = e->B.n_sub;
+  if (s0 + n_sub > e->run.replay_nsubreads)
+    return fail(e, PBSIM_E_REPLAY, "replay log exhausted: batch needs subreads %lld..%lld but the log has %lld",
+                (long long)s0, (long long)(s0 + n_sub), (long long)e->run.replay_nsubreads);
+  const int64_t d0 = e->run.replay_starts[s0];
+  const int64_t d1 = (s0 + n_sub < e->run.replay_nsubreads) ? e->run.replay_starts[s0 + n_sub] : e->run.replay_ndraws;
+  c.next_start_after = (s0 + n_sub < e->run.replay_nsubreads) ? d1 : e->run.replay_ndraws;
+  if (d0 < 0 || d1 < d0 || d1 > e->run.replay_ndraws) return fail(e, PBSIM_E_REPLAY, "replay starts are not monotone");
+  if (upload(e, e->d_draws, e->run.replay_draws + d0, (size_t)(d1 - d0))) return PBSIM_E_CUDA;
+  if (upload(e, e->d_starts, e->run.replay_starts + s0, (size_t)n_sub)) return PBSIM_E_CUDA;
+  c.A.rng.draws = e->d_draws.as<int32_t>();
+  c.A.rng.draws_base = d0;
+  c.A.rng.draws_end = d1;
+  c.A.rng.starts = e->d_starts.as<int64_t>();
+  return 0;
+}
+
+// K1 plan, then the pass-1 schedule: sub-reads sorted by (accuracy, length desc), longest-first CTA order
+int plan(pbsim_engine *e, BatchCtx &c) {
   Batch &B = e->B;
-  const uint32_t n_sub = B.n_sub;
-  B.first_read = (uint64_t)e->next_read;
-  const uint32_t cta_threads = qs ? kSimThreads : kErrThreads;
-  const uint32_t cta_slots = nblk(n_sub, cta_threads) + kBins;
-  CK(e->d_bins.ensure((4 * kBins + 8) * 4 + (size_t)cta_slots * 4 * 4));
-  CK(e->d_ctrl.ensure(64 * 8));
-  CK(e->h_ctrl.ensure(64 * 8));
-  uint32_t *bin_start = e->d_bins.as<uint32_t>();
-  uint32_t *bin_lo = bin_start + kBins + 1, *bin_hi = bin_lo + kBins, *cta_first = bin_hi + kBins;
-  uint32_t *cta_key = cta_first + kBins + 1, *cta_id = cta_key + cta_slots, *cta_key_s = cta_id + cta_slots,
-           *cta_order = cta_key_s + cta_slots;
-  unsigned long long *ctrl = e->d_ctrl.as<unsigned long long>();
-  unsigned long long *hctrl = reinterpret_cast<unsigned long long *>(e->h_ctrl.p);
+  const uint32_t seg_min_len = c.use_segments ? (uint32_t)e->seg_min_len : 0u;
+  if (c.sample)
+    k_plan_sample<<<nblk(B.n_reads, 256), 256, 0, e->st>>>(c.A.G, c.Pl, *c.sb, B, e->cap_num, e->cap_den, c.spec ? 1u : 0u,
+                                                             c.A.rng.seed, c.A.M.uniform_bias ? 1u : 0u, seg_min_len);
+  else
+    k_plan<<<nblk(B.n_reads, 256), 256, 0, e->st>>>(c.A.M, c.A.G, device_set(e), c.A.rng, B, c.clip_room, e->cap_num,
+                                                      e->cap_den, c.qs ? 8u : 16u, seg_min_len, e->seg_extra,
+                                                      e->chain_chunk_eff());
+  e->launches++;
+  return schedule_ctas(e, e->d_bins, B.key_in, B.key_out, B.idx_in, B.order, B.n_sub, 0, c.cta_threads, true, &c.cta);
+}
 
-  DeviceModel M = device_model(e);
-  DeviceGenome G = device_genome(e);
-  RngParams rng;
-  rng.mode = (uint32_t)e->run.rng_mode;
-  rng.seed = e->run.seed;
-  rng.draws = nullptr;
-  rng.draws_base = 0;
-  rng.draws_end = 0;
-  rng.starts = nullptr;
-  int64_t next_start_after = -1;
-  if (replay) {
-    // upload the slice of the draw log this batch can touch
-    const int64_t s0 = (int64_t)(e->next_read - e->run.first_read) * pass;
-    if (s0 + (int64_t)n_sub > e->run.replay_nsubreads)
-      return fail(e, PBSIM_E_REPLAY, "replay log exhausted: batch needs subreads %lld..%lld but the log has %lld",
-                  (long long)s0, (long long)(s0 + n_sub), (long long)e->run.replay_nsubreads);
-    const int64_t d0 = e->run.replay_starts[s0];
-    const int64_t d1 = (s0 + n_sub < e->run.replay_nsubreads) ? e->run.replay_starts[s0 + n_sub] : e->run.replay_ndraws;
-    next_start_after = (s0 + n_sub < e->run.replay_nsubreads) ? d1 : e->run.replay_ndraws;
-    if (d0 < 0 || d1 < d0 || d1 > e->run.replay_ndraws) return fail(e, PBSIM_E_REPLAY, "replay starts are not monotone");
-    if (upload(e, e->d_draws, e->run.replay_draws + d0, (size_t)(d1 - d0))) return PBSIM_E_CUDA;
-    if (upload(e, e->d_starts, e->run.replay_starts + s0, (size_t)n_sub)) return PBSIM_E_CUDA;
-    rng.draws = e->d_draws.as<int32_t>();
-    rng.draws_base = d0;
-    rng.draws_end = d1;
-    rng.starts = e->d_starts.as<int64_t>();
+// event and checkpoint slots, and with segments the segment and chunk lists: offsets by scans, totals read back
+int size_slots(pbsim_engine *e, BatchCtx &c) {
+  Batch &B = e->B;
+  unsigned long long *hctrl = host_ctrl(e);
+  unsigned long long *tmp = u64_slice(e, kSliceScanIn);
+  unsigned long long *seg_off = u64_slice(e, kSliceSegOff), *chunk_off = u64_slice(e, kSliceChunkOff);
+  int rc;
+  if ((rc = widen_scan(e, B.cap, B.n_sub, tmp, reinterpret_cast<unsigned long long *>(B.ev_off)))) return rc;
+  if ((rc = widen_scan(e, B.ck_cap, B.n_sub, tmp, reinterpret_cast<unsigned long long *>(B.ck_off)))) return rc;
+  if (c.use_segments) {
+    if ((rc = widen_scan(e, B.nseg, B.n_sub, tmp, seg_off))) return rc;
+    if (peek(e, hctrl + 2, seg_off + B.n_sub, 8)) return PBSIM_E_CUDA;
+    if ((rc = widen_scan(e, B.nchunk, B.n_sub, tmp, chunk_off))) return rc;
+    if (peek(e, hctrl + 4, chunk_off + B.n_sub, 8)) return PBSIM_E_CUDA;
   }
+  if (peek(e, hctrl, B.ev_off + B.n_sub, 8)) return PBSIM_E_CUDA;
+  if (peek(e, hctrl + 1, B.ck_off + B.n_sub, 8)) return PBSIM_E_CUDA;
+  CK(cudaStreamSynchronize(e->st));
+  c.n_seg_total = c.use_segments ? hctrl[2] : 0;
+  c.n_chunk_total = c.use_segments ? hctrl[4] : 0;
+  if (c.n_seg_total > 0x7FFFFFF0ull) return fail(e, PBSIM_E_INVALID, "too many segments in one batch");
+  CK(e->d_ev.ensure((size_t)hctrl[0] * (c.qs ? 2 : 1) + 256));
+  CK(e->d_ck.ensure((size_t)hctrl[1] * sizeof(Ckpt) + 256));
+  if (c.n_seg_total > 0) CK(e->d_seg.ensure((size_t)c.n_seg_total * (6 * 4 + sizeof(SegResult)) + 256));
+  return 0;
+}
 
-  // (the single, quota-clipped read of a tail batch is segmented too: on one thread a 50 kb read takes milliseconds)
-  // (--method sample: the speculative pass of PHILOX runs; the chains that have to be redone stay sequential)
-  bool use_segments = !replay && e->seg_enabled && (!sample || spec);
-  int seg_retries = 0;
-  for (int attempt = 0; attempt < 9; ++attempt) {
-    // ---- K1 plan
-    const uint32_t ev_align = qs ? 8u : 16u;
-    if (sample)
-      k_plan_sample<<<nblk(n_reads, 256), 256, 0, e->st>>>(G, Pl, *sb, B, e->cap_num, e->cap_den, spec ? 1u : 0u, rng.seed,
-                                                           M.uniform_bias ? 1u : 0u,
-                                                           use_segments ? (uint32_t)e->seg_min_len : 0u);
-    else
-      k_plan<<<nblk(n_reads, 256), 256, 0, e->st>>>(M, G, device_set(e), rng, B, clip_room, e->cap_num, e->cap_den, ev_align,
-                                                     use_segments ? (uint32_t)e->seg_min_len : 0u, e->seg_extra,
-                                                     e->chain_chunk_eff());
-    e->launches++;
-    // ---- sort by (accuracy, length desc), bins, longest-first CTA order
-    auto schedule = [&]() -> int {
-      {
-        size_t tmp = 0;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, B.key_in, B.key_out, B.idx_in, B.order, (int)n_sub, 0, 28, e->st));
-        CK(e->d_cub_tmp.ensure(tmp + 256));
-        tmp = e->d_cub_tmp.cap;
-        CK(cub::DeviceRadixSort::SortPairs(e->d_cub_tmp.p, tmp, B.key_in, B.key_out, B.idx_in, B.order, (int)n_sub, 0, 28,
-                                           e->st));
-      }
-      k_fill_u32<<<1, 256, 0, e->st>>>(bin_start, kBins + 1, 0xFFFFFFFFu);
-      k_bin_bounds<<<nblk(n_sub, 256), 256, 0, e->st>>>(B.key_out, n_sub, bin_start);
-      k_cta_map<<<1, 32, 0, e->st>>>(bin_start, B.key_out, n_sub, bin_lo, bin_hi, cta_first, cta_threads);
-      k_cta_keys<<<nblk(cta_slots, 256), 256, 0, e->st>>>(B.key_out, bin_lo, cta_first, cta_slots, cta_key, cta_id, cta_threads);
-      {
-        size_t tmp = 0;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, cta_key, cta_key_s, cta_id, cta_order, (int)cta_slots, 0, 21, e->st));
-        CK(e->d_cub_tmp.ensure(tmp + 256));
-        tmp = e->d_cub_tmp.cap;
-        CK(cub::DeviceRadixSort::SortPairs(e->d_cub_tmp.p, tmp, cta_key, cta_key_s, cta_id, cta_order, (int)cta_slots, 0, 21,
-                                           e->st));
-      }
-      e->launches += 4;
-      return 0;
-    };
-    if ((rc = schedule())) return rc;
-    // ---- slots
-    unsigned long long *tmp64 = reinterpret_cast<unsigned long long *>(u64_slice(e, 2));
-    k_widen<<<nblk(n_sub + 1, 256), 256, 0, e->st>>>(B.cap, n_sub, tmp64);
-    if ((rc = excl_scan(e, tmp64, reinterpret_cast<unsigned long long *>(B.ev_off), n_sub + 1))) return rc;
-    k_widen<<<nblk(n_sub + 1, 256), 256, 0, e->st>>>(B.ck_cap, n_sub, tmp64);
-    if ((rc = excl_scan(e, tmp64, reinterpret_cast<unsigned long long *>(B.ck_off), n_sub + 1))) return rc;
+// K2 / K3: sequential pass 1, one thread per sub-read
+void pass1_sequential(pbsim_engine *e, BatchCtx &c) {
+  SimArgs &A = c.A;
+  set_ctas(A, c.cta);
+  A.ev = e->d_ev.as<uint8_t>();
+  A.ck = e->d_ck.as<Ckpt>();
+  const uint32_t grid = c.cta.slots;
+  if (c.sample) {
+    if (c.replay) k_sim_sample<PBSIM_RNG_REPLAY><<<grid, kSimThreads, 0, e->st>>>(A, c.Pl, *c.sb, 0u);
+    else k_sim_sample<PBSIM_RNG_PHILOX><<<grid, kSimThreads, 0, e->st>>>(A, c.Pl, *c.sb, 0u);
+  } else if (c.qs) {
+    if (c.replay) k_sim_qshmm<PBSIM_RNG_REPLAY><<<grid, kSimThreads, kQsSmemBytes, e->st>>>(A);
+    else k_sim_qshmm<PBSIM_RNG_PHILOX><<<grid, kSimThreads, kQsSmemBytes, e->st>>>(A);
+  } else {
+    const uint32_t smem = e->er_smem_bar_off + 16;
+    if (c.replay) k_sim_errhmm<PBSIM_RNG_REPLAY><<<grid, kErrThreads, smem, e->st>>>(A, e->er_smem_bar_off);
+    else k_sim_errhmm<PBSIM_RNG_PHILOX><<<grid, kErrThreads, smem, e->st>>>(A, e->er_smem_bar_off);
+  }
+  e->launches++;
+}
+
+// segment-parallel pass 1 for the long reads (seg_kernels.cuh): the chain-only pass computes the HMM state in front of
+// every segment (k_chain_chunk), then the segments run and k_find_end finds where each read ends
+int pass1_segments(pbsim_engine *e, BatchCtx &c) {
+  const Batch &B = e->B;
+  const uint32_t nseg = (uint32_t)c.n_seg_total;
+  SegBatch S;
+  S.n_seg_total = nseg;
+  S.seg_off = reinterpret_cast<const uint64_t *>(u64_slice(e, kSliceSegOff));
+  S.seg_res = e->d_seg.as<SegResult>();
+  uint32_t *u = reinterpret_cast<uint32_t *>(S.seg_res + nseg);
+  uint32_t **seg_arrays[] = {&S.seg_sub, &S.seg_key_in, &S.seg_key_out, &S.seg_id_in, &S.seg_order, &S.seg_state};
+  for (size_t i = 0; i < 6; ++i) *seg_arrays[i] = u + i * nseg;
+  k_seg_fill<<<nblk(B.n_sub, 256), 256, 0, e->st>>>(B, S, c.pass);
+  CtaSchedule sc;
+  int rc = schedule_ctas(e, e->d_seg_bins, S.seg_key_in, S.seg_key_out, S.seg_id_in, S.seg_order, nseg, 20, c.cta_threads,
+                         false, &sc);
+  if (rc) return rc;
+  SegArgs SA;
+  SA.keys = c.A.keys;
+  SA.M = c.A.M;
+  SA.G = c.A.G;
+  SA.bias_one = e->d_biasone.as<uint8_t>();
+  SA.B = B;
+  SA.S = S;
+  set_ctas(SA, sc);
+  SA.ev = e->d_ev.as<uint8_t>();
+  SA.pool_q = c.Pl.quals;
+  SA.pool_start = c.Pl.start;
+  if (c.n_chunk_total > 0) {
+    const uint32_t nch = (uint32_t)c.n_chunk_total;
+    const uint32_t chain_threads = c.qs ? (uint32_t)kChainThreads : c.cta_threads;
+    CK(e->d_chunk.ensure((size_t)nch * 5 * 4 + 64));
+    ChunkBatch C;
+    C.n_chunks = nch;
+    C.per_chunk = e->chain_chunk_eff();
+    C.qs = c.qs ? 1u : 0u;
+    C.chunk_off = reinterpret_cast<const uint64_t *>(u64_slice(e, kSliceChunkOff));
+    uint32_t **chunk_arrays[] = {&C.sub, &C.key_in, &C.key_out, &C.id_in, &C.order};
+    for (size_t i = 0; i < 5; ++i) *chunk_arrays[i] = e->d_chunk.as<uint32_t>() + i * nch;
+    k_chunk_fill<<<nblk(B.n_sub, 256), 256, 0, e->st>>>(B, C, c.pass);
+    CtaSchedule cc;
+    if ((rc = schedule_ctas(e, e->d_chunk_bins, C.key_in, C.key_out, C.id_in, C.order, nch, 0, chain_threads, true, &cc)))
+      return rc;
+    SegArgs CA = SA;
+    set_ctas(CA, cc);
+    CK(cudaEventRecord(e->ev_chain[0], e->st));
+    if (c.qs) k_chain_chunk<<<cc.slots, kChainThreads, kQsSmemBytes, e->st>>>(CA, C);
+    else k_chain_chunk_err<<<cc.slots, kErrThreads, e->er_smem_bar_off + 16, e->st>>>(CA, C, e->er_smem_bar_off);
+    CK(cudaEventRecord(e->ev_chain[1], e->st));
     e->launches += 2;
-    unsigned long long *seg_off = reinterpret_cast<unsigned long long *>(u64_slice(e, 10));
-    unsigned long long *chunk_off = reinterpret_cast<unsigned long long *>(u64_slice(e, 11));
-    hctrl[2] = 0;
-    hctrl[4] = 0;
-    if (use_segments) {
-      k_widen<<<nblk(n_sub + 1, 256), 256, 0, e->st>>>(B.nseg, n_sub, tmp64);
-      if ((rc = excl_scan(e, tmp64, seg_off, n_sub + 1))) return rc;
-      e->launches++;
-      if (peek(e, hctrl + 2, seg_off + n_sub, 8)) return PBSIM_E_CUDA;
-      k_widen<<<nblk(n_sub + 1, 256), 256, 0, e->st>>>(B.nchunk, n_sub, tmp64);
-      if ((rc = excl_scan(e, tmp64, chunk_off, n_sub + 1))) return rc;
-      e->launches++;
-      if (peek(e, hctrl + 4, chunk_off + n_sub, 8)) return PBSIM_E_CUDA;
-    }
-    if (peek(e, hctrl, B.ev_off + n_sub, 8)) return PBSIM_E_CUDA;
-    if (peek(e, hctrl + 1, B.ck_off + n_sub, 8)) return PBSIM_E_CUDA;
-    CK(cudaStreamSynchronize(e->st));
-    const uint64_t ev_entries = hctrl[0], ck_entries = hctrl[1];
-    const uint64_t n_seg_total = use_segments ? hctrl[2] : 0;
-    const uint64_t n_chunk_total = use_segments ? hctrl[4] : 0;
-    if (n_seg_total > 0x7FFFFFF0ull) return fail(e, PBSIM_E_INVALID, "too many segments in one batch");
-    CK(e->d_ev.ensure((size_t)ev_entries * (qs ? 2 : 1) + 256));
-    CK(e->d_ck.ensure((size_t)ck_entries * sizeof(Ckpt) + 256));
-
-    if (n_seg_total > 0) CK(e->d_seg.ensure((size_t)n_seg_total * (6 * 4 + sizeof(SegResult)) + 256));
-    // ---- K2 / K3 pass 1
-    SimArgs A;
-    A.bias_one = e->d_biasone.as<uint8_t>();
-    A.plan_draws = e->strategy == PBSIM_STRATEGY_TRANS ? 3u : (e->strategy == PBSIM_STRATEGY_TEMPL ? 1u : 0u);
-    A.keys.init(rng.seed, (uint32_t)e->seq_num);
-    A.M = M;
-    A.G = G;
-    A.rng = rng;
-    A.B = B;
-    A.cta_order = cta_order;
-    A.cta_first = cta_first;
-    A.bin_lo = bin_lo;
-    A.bin_hi = bin_hi;
-    A.ev = e->d_ev.as<uint8_t>();
-    A.ck = e->d_ck.as<Ckpt>();
-    const uint32_t grid = cta_slots;
-    bool seg_timed = false, chain_timed = false;
-    CK(cudaEventRecord(e->ev_k[0], e->st));
-    if (sample) {
-      if (replay) k_sim_sample<PBSIM_RNG_REPLAY><<<grid, kSimThreads, 0, e->st>>>(A, Pl, *sb, 0u);
-      else k_sim_sample<PBSIM_RNG_PHILOX><<<grid, kSimThreads, 0, e->st>>>(A, Pl, *sb, 0u);
-    } else if (qs) {
-      if (replay) k_sim_qshmm<PBSIM_RNG_REPLAY><<<grid, kSimThreads, kQsSmemBytes, e->st>>>(A);
-      else k_sim_qshmm<PBSIM_RNG_PHILOX><<<grid, kSimThreads, kQsSmemBytes, e->st>>>(A);
-    } else {
-      const uint32_t smem = e->er_smem_bar_off + 16;
-      if (replay) k_sim_errhmm<PBSIM_RNG_REPLAY><<<grid, kErrThreads, smem, e->st>>>(A, e->er_smem_bar_off);
-      else k_sim_errhmm<PBSIM_RNG_PHILOX><<<grid, kErrThreads, smem, e->st>>>(A, e->er_smem_bar_off);
-    }
-    e->launches++;
-    if (n_seg_total > 0) {
-      // ---- segment-parallel pass 1 for the long reads (seg_kernels.cuh)
-      const uint32_t nseg = (uint32_t)n_seg_total;
-      const uint32_t seg_slots = nblk(nseg, cta_threads) + kBins;
-      CK(e->d_seg_bins.ensure((4 * kBins + 8) * 4 + (size_t)seg_slots * 4 + 64));
-      SegBatch S;
-      S.n_seg_total = nseg;
-      S.seg_off = (const uint64_t *)seg_off;
-      S.seg_res = e->d_seg.as<SegResult>();
-      uint32_t *u = reinterpret_cast<uint32_t *>(S.seg_res + nseg);
-      S.seg_sub = u;
-      S.seg_key_in = u + nseg;
-      S.seg_key_out = u + 2ull * nseg;
-      S.seg_id_in = u + 3ull * nseg;
-      S.seg_order = u + 4ull * nseg;
-      S.seg_state = u + 5ull * nseg;
-      uint32_t *sb_start = e->d_seg_bins.as<uint32_t>();
-      uint32_t *sb_lo = sb_start + kBins + 1, *sb_hi = sb_lo + kBins, *sb_first = sb_hi + kBins, *sb_order = sb_first + kBins + 1;
-      k_seg_fill<<<nblk(n_sub, 256), 256, 0, e->st>>>(B, S, pass);
-      {
-        size_t tmp = 0;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, S.seg_key_in, S.seg_key_out, S.seg_id_in, S.seg_order, (int)nseg, 20,
-                                           28, e->st));
-        CK(e->d_cub_tmp.ensure(tmp + 256));
-        tmp = e->d_cub_tmp.cap;
-        CK(cub::DeviceRadixSort::SortPairs(e->d_cub_tmp.p, tmp, S.seg_key_in, S.seg_key_out, S.seg_id_in, S.seg_order,
-                                           (int)nseg, 20, 28, e->st));
-      }
-      k_fill_u32<<<1, 256, 0, e->st>>>(sb_start, kBins + 1, 0xFFFFFFFFu);
-      k_bin_bounds<<<nblk(nseg, 256), 256, 0, e->st>>>(S.seg_key_out, nseg, sb_start);
-      k_cta_map<<<1, 32, 0, e->st>>>(sb_start, S.seg_key_out, nseg, sb_lo, sb_hi, sb_first, cta_threads);
-      k_iota_u32<<<nblk(seg_slots, 256), 256, 0, e->st>>>(sb_order, seg_slots);
-      SegArgs SA;
-      SA.keys = A.keys;
-      SA.M = M;
-      SA.G = G;
-      SA.bias_one = e->d_biasone.as<uint8_t>();
-      SA.B = B;
-      SA.S = S;
-      SA.cta_order = sb_order;
-      SA.cta_first = sb_first;
-      SA.bin_lo = sb_lo;
-      SA.bin_hi = sb_hi;
-      SA.ev = e->d_ev.as<uint8_t>();
-      SA.pool_q = Pl.quals;
-      SA.pool_start = Pl.start;
-      if (n_chunk_total > 0) {
-        // ---- chain-only pass: the HMM state in front of every segment (k_chain_chunk), scheduled like the segments
-        const uint32_t nch = (uint32_t)n_chunk_total;
-        const uint32_t chain_threads = qs ? (uint32_t)kChainThreads : cta_threads;
-        const uint32_t ch_slots = nblk(nch, chain_threads) + kBins;
-        CK(e->d_chunk.ensure((size_t)nch * 5 * 4 + 64));
-        CK(e->d_chunk_bins.ensure((4 * kBins + 8) * 4 + (size_t)ch_slots * 4 * 4 + 64));
-        ChunkBatch C;
-        C.n_chunks = nch;
-        C.per_chunk = e->chain_chunk_eff();
-        C.qs = qs ? 1u : 0u;
-        C.chunk_off = (const uint64_t *)chunk_off;
-        uint32_t *cu = e->d_chunk.as<uint32_t>();
-        C.sub = cu;
-        C.key_in = cu + nch;
-        C.key_out = cu + 2ull * nch;
-        C.id_in = cu + 3ull * nch;
-        C.order = cu + 4ull * nch;
-        uint32_t *cb_start = e->d_chunk_bins.as<uint32_t>();
-        uint32_t *cb_lo = cb_start + kBins + 1, *cb_hi = cb_lo + kBins, *cb_first = cb_hi + kBins;
-        uint32_t *cb_key = cb_first + kBins + 1, *cb_id = cb_key + ch_slots, *cb_key_s = cb_id + ch_slots,
-                 *cb_order = cb_key_s + ch_slots;
-        k_chunk_fill<<<nblk(n_sub, 256), 256, 0, e->st>>>(B, C, pass);
-        {
-          size_t tmp = 0;
-          CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, C.key_in, C.key_out, C.id_in, C.order, (int)nch, 0, 28, e->st));
-          CK(e->d_cub_tmp.ensure(tmp + 256));
-          tmp = e->d_cub_tmp.cap;
-          CK(cub::DeviceRadixSort::SortPairs(e->d_cub_tmp.p, tmp, C.key_in, C.key_out, C.id_in, C.order, (int)nch, 0, 28, e->st));
-        }
-        k_fill_u32<<<1, 256, 0, e->st>>>(cb_start, kBins + 1, 0xFFFFFFFFu);
-        k_bin_bounds<<<nblk(nch, 256), 256, 0, e->st>>>(C.key_out, nch, cb_start);
-        k_cta_map<<<1, 32, 0, e->st>>>(cb_start, C.key_out, nch, cb_lo, cb_hi, cb_first, chain_threads);
-        k_cta_keys<<<nblk(ch_slots, 256), 256, 0, e->st>>>(C.key_out, cb_lo, cb_first, ch_slots, cb_key, cb_id, chain_threads);
-        {
-          size_t tmp = 0;
-          CK(cub::DeviceRadixSort::SortPairs(nullptr, tmp, cb_key, cb_key_s, cb_id, cb_order, (int)ch_slots, 0, 21, e->st));
-          CK(e->d_cub_tmp.ensure(tmp + 256));
-          tmp = e->d_cub_tmp.cap;
-          CK(cub::DeviceRadixSort::SortPairs(e->d_cub_tmp.p, tmp, cb_key, cb_key_s, cb_id, cb_order, (int)ch_slots, 0, 21, e->st));
-        }
-        SegArgs CA = SA;
-        CA.cta_order = cb_order;
-        CA.cta_first = cb_first;
-        CA.bin_lo = cb_lo;
-        CA.bin_hi = cb_hi;
-        static bool chain_carve = false;
-        if (!chain_carve) {
-          CK(cudaFuncSetAttribute(k_chain_chunk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-          chain_carve = true;
-        }
-        CK(cudaEventRecord(e->ev_chain[0], e->st));
-        if (qs) k_chain_chunk<<<ch_slots, kChainThreads, kQsSmemBytes, e->st>>>(CA, C);
-        else k_chain_chunk_err<<<ch_slots, kErrThreads, e->er_smem_bar_off + 16, e->st>>>(CA, C, e->er_smem_bar_off);
-        CK(cudaEventRecord(e->ev_chain[1], e->st));
-        chain_timed = true;
-        e->launches += 6;
-      }
-      CK(cudaEventRecord(e->ev_seg[0], e->st));
-      seg_timed = true;
-      if (qs) {
-        if (sample) k_sim_seg<true><<<seg_slots, kSimThreads, 0, e->st>>>(SA);
-        else k_sim_seg<false><<<seg_slots, kSimThreads, 0, e->st>>>(SA);
-        CK(cudaEventRecord(e->ev_seg[1], e->st));
-        k_find_end<<<nblk((uint64_t)n_sub * 32, 128), 128, 0, e->st>>>(B, S, G, e->d_biasone.as<uint8_t>(), pass,
-                                                                       e->d_ev.as<uint8_t>(), e->d_ck.as<Ckpt>(), M.qs_fast,
-                                                                       sample ? 1u : 0u);
-      } else {
-        k_sim_seg_err<<<seg_slots, kErrThreads, e->er_smem_bar_off + 16, e->st>>>(SA, e->er_smem_bar_off);
-        CK(cudaEventRecord(e->ev_seg[1], e->st));
-        k_find_end_err<<<nblk((uint64_t)n_sub * 32, 128), 128, 0, e->st>>>(B, S, G, SA.keys, e->d_biasone.as<uint8_t>(), pass,
-                                                                           e->d_ev.as<uint8_t>(), e->d_ck.as<Ckpt>());
-      }
-      e->launches += 7;
-      e->seg_batches++;
-    }
-    if (sample && spec) {
-      // which copies assumed a wrong length?  Their groups' tails are redone as chains (k_sample_redo), one thread per
-      // chain, in the sequential slot layout (k_sim_sample clears the reads' "segmented" mark)
-      hctrl[6] = 0;
-      CK(cudaMemsetAsync(ctrl + 6, 0, 8, e->st));
-      k_sample_redo<<<nblk(n_reads, 256), 256, 0, e->st>>>(B, ctrl + 6);
-      if (peek(e, hctrl + 6, ctrl + 6, 8)) return PBSIM_E_CUDA;
-      CK(cudaStreamSynchronize(e->st));
-      e->launches += 2;
-      if (hctrl[6] > 0) {
-        if ((rc = schedule())) return rc;
-        if (replay) k_sim_sample<PBSIM_RNG_REPLAY><<<grid, kSimThreads, 0, e->st>>>(A, Pl, *sb, 1u);
-        else k_sim_sample<PBSIM_RNG_PHILOX><<<grid, kSimThreads, 0, e->st>>>(A, Pl, *sb, 1u);
-        e->launches++;
-        e->sample_redo_groups += (int64_t)hctrl[6];
-        if (hctrl[6] * 2 > sb->n_groups) e->sample_spec_run = false;  // deletion-rich mix: chains from the start
-      }
-    }
-    CK(cudaEventRecord(e->ev_k[1], e->st));
-    CK(cudaGetLastError());
-
-    // ---- quota: which read crosses len_quota
-    unsigned long long *rl0 = reinterpret_cast<unsigned long long *>(u64_slice(e, 2));
-    unsigned long long *prefix = reinterpret_cast<unsigned long long *>(u64_slice(e, 3));
-    k_rlen0<<<nblk(n_reads, 256), 256, 0, e->st>>>(B.rlen, n_reads, pass, rl0);
-    if ((rc = excl_scan(e, rl0, prefix, n_reads))) return rc;
-    hctrl[0] = n_reads;
-    hctrl[1] = 0;
-    hctrl[2] = 0;
-    hctrl[3] = 0;
-    CK(cudaMemcpyAsync(ctrl, hctrl, 32, cudaMemcpyHostToDevice, e->st));
-    if (sample)
-      k_find_cut_sample<<<nblk(n_reads, 256), 256, 0, e->st>>>(prefix, n_reads, e->len_total, e->run.len_quota, ctrl);
-    else if (clip_room < 0)  // bulk batch: speculative unclipped plans
-      k_find_cut<<<nblk(n_reads, 256), 256, 0, e->st>>>(prefix, B.plan_raw, n_reads, e->len_total, e->run.len_quota, ctrl);
-    k_batch_totals<<<nblk(n_sub, 256), 256, 0, e->st>>>(prefix, B.rlen, B.flags, n_reads, pass, ctrl);
-    e->launches += 3;
-    if (replay) {
-      k_check_replay<<<nblk(n_sub, 256), 256, 0, e->st>>>(rng.starts, B.draws_used, B.plan_wlen, (uint32_t)e->glen, n_sub,
-                                                          pass, next_start_after, ctrl, reinterpret_cast<unsigned int *>(&ctrl[3]));
-      e->launches++;
-    }
-    if (peek(e, hctrl, ctrl, 32)) return PBSIM_E_CUDA;
-    CK(cudaStreamSynchronize(e->st));
-    const uint32_t flags = (uint32_t)hctrl[2];
-    if (flags & 2u) return fail(e, PBSIM_E_PARAM, "a read drew an accuracy for which the model has no usable tables");
-    {
-      float ms = 0;
-      CK(cudaEventElapsedTime(&ms, e->ev_k[0], e->ev_k[1]));
-      e->sim_ms += ms;
-      if (seg_timed) {
-        CK(cudaEventElapsedTime(&ms, e->ev_seg[0], e->ev_seg[1]));
-        e->seg_ms += ms;
-      }
-      if (chain_timed) {
-        CK(cudaEventElapsedTime(&ms, e->ev_chain[0], e->ev_chain[1]));
-        e->chain_ms += ms;
-      }
-    }
-    if (getenv("PBSIM_DEBUG")) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, e->ev_k[0], e->ev_k[1]);
-      fprintf(stderr, "[pbsim] batch reads=%u sub=%u segments=%llu flags=%u pass1_ms=%.2f attempt=%d\n", n_reads, n_sub,
-              (unsigned long long)n_seg_total, flags, ms, attempt);
-    }
-    if (flags & 4u) {
-      // A segmented read could not be completed.  If the only reason is that its window outlasted the segments
-      // provisioned for it (a read that stays in an insertion-rich state of a sticky chain), provision more — the
-      // headroom stays for the batches to come; anything else redoes the batch on the sequential path.
-      const uint32_t inner = flags >> 8;
-      if (inner == 4u && e->seg_extra < 0.6f && seg_retries < 3) {
-        e->seg_extra += 0.04f;
-        ++seg_retries;
-        continue;
-      }
-      use_segments = false;
-      e->seg_fallback_batches++;
-      if (attempt >= 8) return fail(e, PBSIM_E_OVERFLOW, "segment-parallel pass 1 failed repeatedly");
-      continue;
-    }
-    if (flags & 1u) {  // a read outgrew its slot: enlarge and redo the batch
-      e->cap_num *= 2;
-      if (attempt >= 8) return fail(e, PBSIM_E_OVERFLOW, "event slots overflowed repeatedly");
-      continue;
-    }
-    const uint64_t cut = hctrl[0];
-    out->cut = cut < n_reads;
-    out->n_valid_reads = out->cut ? (uint32_t)cut : n_reads;
-    out->bases_pass0 = hctrl[1];
-    if (replay && hctrl[3] != 0)
-      return fail(e, PBSIM_E_REPLAY, "replay: %llu subreads consumed a different number of draws than the log says",
-                  (unsigned long long)hctrl[3]);
-    break;
   }
+  CK(cudaEventRecord(e->ev_seg[0], e->st));
+  const uint32_t end_grid = nblk((uint64_t)B.n_sub * 32, 128);
+  if (c.qs) {
+    if (c.sample) k_sim_seg<true><<<sc.slots, kSimThreads, 0, e->st>>>(SA);
+    else k_sim_seg<false><<<sc.slots, kSimThreads, 0, e->st>>>(SA);
+    CK(cudaEventRecord(e->ev_seg[1], e->st));
+    k_find_end<<<end_grid, 128, 0, e->st>>>(B, S, c.A.G, SA.bias_one, c.pass, SA.ev, e->d_ck.as<Ckpt>(), c.A.M.qs_fast,
+                                            c.sample ? 1u : 0u);
+  } else {
+    k_sim_seg_err<<<sc.slots, kErrThreads, e->er_smem_bar_off + 16, e->st>>>(SA, e->er_smem_bar_off);
+    CK(cudaEventRecord(e->ev_seg[1], e->st));
+    k_find_end_err<<<end_grid, 128, 0, e->st>>>(B, S, c.A.G, SA.keys, SA.bias_one, c.pass, SA.ev, e->d_ck.as<Ckpt>());
+  }
+  e->launches += 3;
+  e->seg_batches++;
+  return 0;
+}
 
-  const uint32_t nv_sub = out->n_valid_reads * pass;
-  out->reads_bytes = out->maf_bytes = 0;
-  out->bases_all = 0;
+// --method sample: which copies assumed a wrong length?  Their groups' tails are redone as chains (k_sample_redo), one
+// thread per chain, in the sequential slot layout (k_sim_sample clears the reads' "segmented" mark)
+int sample_redo(pbsim_engine *e, BatchCtx &c) {
+  Batch &B = e->B;
+  unsigned long long *ctrl = e->d_ctrl.as<unsigned long long>(), *hctrl = host_ctrl(e);
+  hctrl[6] = 0;
+  CK(cudaMemsetAsync(ctrl + 6, 0, 8, e->st));
+  k_sample_redo<<<nblk(B.n_reads, 256), 256, 0, e->st>>>(B, ctrl + 6);
+  if (peek(e, hctrl + 6, ctrl + 6, 8)) return PBSIM_E_CUDA;
+  CK(cudaStreamSynchronize(e->st));
+  e->launches += 2;
+  if (hctrl[6] == 0) return 0;
+  const int rc =
+      schedule_ctas(e, e->d_bins, B.key_in, B.key_out, B.idx_in, B.order, B.n_sub, 0, c.cta_threads, true, &c.cta);
+  if (rc) return rc;
+  if (c.replay) k_sim_sample<PBSIM_RNG_REPLAY><<<c.cta.slots, kSimThreads, 0, e->st>>>(c.A, c.Pl, *c.sb, 1u);
+  else k_sim_sample<PBSIM_RNG_PHILOX><<<c.cta.slots, kSimThreads, 0, e->st>>>(c.A, c.Pl, *c.sb, 1u);
+  e->launches++;
+  e->sample_redo_groups += (int64_t)hctrl[6];
+  if (hctrl[6] * 2 > c.sb->n_groups) e->sample_spec_run = false;  // deletion-rich mix: chains from the start
+  return 0;
+}
+
+// which read crosses len_quota: waits for pass 1 and reads back hctrl[0] the cut, [1] the pass-0 bases in front of
+// it, [2] the pass-1 flags, [3] replay: the subreads whose draws disagree with the log
+int quota_cut(pbsim_engine *e, BatchCtx &c, int attempt) {
+  const Batch &B = e->B;
+  const uint32_t n_reads = B.n_reads, n_sub = B.n_sub;
+  unsigned long long *ctrl = e->d_ctrl.as<unsigned long long>(), *hctrl = host_ctrl(e);
+  unsigned long long *rl0 = u64_slice(e, kSliceScanIn);
+  unsigned long long *prefix = u64_slice(e, kSliceRlen0Prefix);
+  k_rlen0<<<nblk(n_reads, 256), 256, 0, e->st>>>(B.rlen, n_reads, c.pass, rl0);
+  const int rc = excl_scan(e, rl0, prefix, n_reads);
+  if (rc) return rc;
+  hctrl[0] = n_reads;
+  hctrl[1] = 0;
+  hctrl[2] = 0;
+  hctrl[3] = 0;
+  CK(cudaMemcpyAsync(ctrl, hctrl, 32, cudaMemcpyHostToDevice, e->st));
+  if (c.sample)
+    k_find_cut_sample<<<nblk(n_reads, 256), 256, 0, e->st>>>(prefix, n_reads, e->len_total, e->run.len_quota, ctrl);
+  else if (c.clip_room < 0)  // bulk batch: speculative unclipped plans
+    k_find_cut<<<nblk(n_reads, 256), 256, 0, e->st>>>(prefix, B.plan_raw, n_reads, e->len_total, e->run.len_quota, ctrl);
+  k_batch_totals<<<nblk(n_sub, 256), 256, 0, e->st>>>(prefix, B.rlen, B.flags, n_reads, c.pass, ctrl);
+  e->launches += 3;
+  if (c.replay) {
+    k_check_replay<<<nblk(n_sub, 256), 256, 0, e->st>>>(c.A.rng.starts, B.draws_used, B.plan_wlen, (uint32_t)e->glen, n_sub,
+                                                        c.pass, c.next_start_after, ctrl,
+                                                        reinterpret_cast<unsigned int *>(&ctrl[3]));
+    e->launches++;
+  }
+  if (peek(e, hctrl, ctrl, 32)) return PBSIM_E_CUDA;
+  CK(cudaStreamSynchronize(e->st));
+  const uint32_t flags = (uint32_t)hctrl[2];
+  if (flags & 2u) return fail(e, PBSIM_E_PARAM, "a read drew an accuracy for which the model has no usable tables");
+  float pass1_ms = 0, ms = 0;
+  CK(cudaEventElapsedTime(&pass1_ms, e->ev_k[0], e->ev_k[1]));
+  e->sim_ms += pass1_ms;
+  if (c.n_seg_total > 0) {
+    CK(cudaEventElapsedTime(&ms, e->ev_seg[0], e->ev_seg[1]));
+    e->seg_ms += ms;
+    if (c.n_chunk_total > 0) {
+      CK(cudaEventElapsedTime(&ms, e->ev_chain[0], e->ev_chain[1]));
+      e->chain_ms += ms;
+    }
+  }
+  if (getenv("PBSIM_DEBUG"))
+    fprintf(stderr, "[pbsim] batch reads=%u sub=%u segments=%llu flags=%u pass1_ms=%.2f attempt=%d\n", n_reads, n_sub,
+            (unsigned long long)c.n_seg_total, flags, pass1_ms, attempt);
+  return 0;
+}
+
+// K4 record sizes, offsets and text of the reads before the cut, K6 their statistics, and the read-back of their
+// accuracies and lengths
+int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
+  const Batch &B = e->B;
+  const uint32_t nv_sub = out->n_valid_reads * c.pass;
   if (nv_sub == 0) return 0;
+  unsigned long long *hctrl = host_ctrl(e);
 
   // ---- K4 sizes + offsets
-  unsigned long long *reads_size = reinterpret_cast<unsigned long long *>(u64_slice(e, 4));
-  unsigned long long *maf_size = reinterpret_cast<unsigned long long *>(u64_slice(e, 5));
-  unsigned long long *ntiles = reinterpret_cast<unsigned long long *>(u64_slice(e, 6));
-  unsigned long long *reads_off = reinterpret_cast<unsigned long long *>(u64_slice(e, 7));
-  unsigned long long *maf_off = reinterpret_cast<unsigned long long *>(u64_slice(e, 8));
-  unsigned long long *tile_start = reinterpret_cast<unsigned long long *>(u64_slice(e, 9));
+  unsigned long long *reads_size = u64_slice(e, kSliceReadsSize);
+  unsigned long long *maf_size = u64_slice(e, kSliceMafSize);
+  unsigned long long *ntiles = u64_slice(e, kSliceNtiles);
+  unsigned long long *reads_off = u64_slice(e, kSliceReadsOff);
+  unsigned long long *maf_off = u64_slice(e, kSliceMafOff);
+  unsigned long long *tile_start = u64_slice(e, kSliceTileStart);
   CK(cudaMemsetAsync(reads_size + nv_sub, 0, 8, e->st));
   CK(cudaMemsetAsync(maf_size + nv_sub, 0, 8, e->st));
   CK(cudaMemsetAsync(ntiles + nv_sub, 0, 8, e->st));
   e->emitp.glen = (uint32_t)e->glen;
   e->emitp.sam = e->model.pass_num > 1 ? (e->bam ? 2u : 1u) : 0u;
-  e->emitp.qs_segments = qs ? 1u : 0u;
-  e->emitp.sample = sample ? 1u : 0u;
+  e->emitp.qs_segments = c.qs ? 1u : 0u;
+  e->emitp.sample = c.sample ? 1u : 0u;
   {
     char head[192];
     if (e->strategy == PBSIM_STRATEGY_WGS) snprintf(head, sizeof head, "%s%d", e->model.id_prefix, e->seq_num);
@@ -970,6 +914,7 @@ int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult 
   k_sizes<<<nblk(nv_sub, 256), 256, 0, e->st>>>(B, e->emitp, device_set(e), nv_sub, (uint64_t *)reads_size, (uint64_t *)maf_size,
                                                 (uint64_t *)ntiles, e->d_lay.as<EmitLay>());
   e->launches++;
+  int rc;
   if ((rc = excl_scan(e, reads_size, reads_off, nv_sub + 1))) return rc;
   if ((rc = excl_scan(e, maf_size, maf_off, nv_sub + 1))) return rc;
   if ((rc = excl_scan(e, ntiles, tile_start, nv_sub + 1))) return rc;
@@ -987,7 +932,7 @@ int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult 
   // ---- K4 emit
   EmitArgs EA;
   EA.S = device_set(e);
-  EA.G = G;
+  EA.G = c.A.G;
   EA.B = B;
   EA.P = e->emitp;
   EA.ev = e->d_ev.as<uint8_t>();
@@ -1003,7 +948,7 @@ int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult 
   EA.reads_off = (const uint64_t *)reads_off;
   EA.maf_off = (const uint64_t *)maf_off;
   EA.keys.init(e->run.seed, (uint32_t)e->seq_num);
-  EA.philox = replay ? 0u : 1u;
+  EA.philox = c.replay ? 0u : 1u;
   EA.out_reads = O.reads.as<uint8_t>();
   EA.out_maf = O.maf.as<uint8_t>();
   if (n_tiles > 0) {
@@ -1011,29 +956,23 @@ int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult 
     cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, e->device);
     const uint64_t want = (n_tiles + kEmitWarps - 1) / kEmitWarps;
     const uint32_t grid = (uint32_t)std::min<uint64_t>(want, (uint64_t)dev_sms * 8 * 4);
-    static bool carve_set = false;
-    if (!carve_set) {  // the staging rows need shared memory for 4 CTAs per SM: ask for the largest carve-out
-      CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_QSHMM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_ERRHMM>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      carve_set = true;
-    }
     CK(cudaEventRecord(e->ev_k[2], e->st));
     // per-tile descriptors (and the tile -> sub-read map), then the row kernel on the plain text tiles and
     // k_emit on everything else (headers, exceptional / wide tiles, SAM arrays, BAM records)
-    if (qs) k_tile_desc<PBSIM_METHOD_QSHMM><<<nblk(n_tiles, 256), 256, 0, e->st>>>(EA, e->d_tile_sub.as<uint32_t>());
+    if (c.qs) k_tile_desc<PBSIM_METHOD_QSHMM><<<nblk(n_tiles, 256), 256, 0, e->st>>>(EA, e->d_tile_sub.as<uint32_t>());
     else k_tile_desc<PBSIM_METHOD_ERRHMM><<<nblk(n_tiles, 256), 256, 0, e->st>>>(EA, e->d_tile_sub.as<uint32_t>());
     e->launches++;
     if (EA.P.sam == 2u) {  // BAM packs bases with atomic ORs: the records start zeroed
       CK(cudaMemsetAsync(O.reads.p, 0, (size_t)out->reads_bytes, e->st));
-      if (qs) k_emit<PBSIM_METHOD_QSHMM, true><<<grid, kEmitThreads, 0, e->st>>>(EA);
+      if (c.qs) k_emit<PBSIM_METHOD_QSHMM, true><<<grid, kEmitThreads, 0, e->st>>>(EA);
       else k_emit<PBSIM_METHOD_ERRHMM, true><<<grid, kEmitThreads, 0, e->st>>>(EA);
     } else {
       const uint32_t glen_words = (uint32_t)((e->glen + 15) / 16);
-      if (qs) {
-        k_emit_rows<PBSIM_METHOD_QSHMM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, n_tiles, EA.ev, G.pk, glen_words, EA.out_reads, EA.out_maf);
+      if (c.qs) {
+        k_emit_rows<PBSIM_METHOD_QSHMM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, n_tiles, EA.ev, c.A.G.pk, glen_words, EA.out_reads, EA.out_maf);
         k_emit<PBSIM_METHOD_QSHMM, false><<<grid, kEmitThreads, 0, e->st>>>(EA);
       } else {
-        k_emit_rows<PBSIM_METHOD_ERRHMM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, n_tiles, EA.ev, G.pk, glen_words, EA.out_reads, EA.out_maf);
+        k_emit_rows<PBSIM_METHOD_ERRHMM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, n_tiles, EA.ev, c.A.G.pk, glen_words, EA.out_reads, EA.out_maf);
         k_emit<PBSIM_METHOD_ERRHMM, false><<<grid, kEmitThreads, 0, e->st>>>(EA);
       }
       e->launches++;
@@ -1042,7 +981,7 @@ int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult 
     e->launches++;
   }
   // ---- K6 stats
-  k_stats<<<nblk(nv_sub, 256), 256, 0, e->st>>>(B, nv_sub, pass, e->d_stats.as<unsigned long long>(), e->freq_len_cells);
+  k_stats<<<nblk(nv_sub, 256), 256, 0, e->st>>>(B, nv_sub, c.pass, e->d_stats.as<unsigned long long>(), e->freq_len_cells);
   e->launches++;
   CK(cudaGetLastError());
 
@@ -1055,9 +994,90 @@ int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult 
   return 0;
 }
 
+// sb: --method sample, the groups of this batch (n_reads = their copies); otherwise null
+int run_batch(pbsim_engine *e, uint32_t n_reads, int64_t clip_room, BatchResult *out, const SampleBatch *sb = nullptr) {
+  BatchCtx c = {};
+  c.pass = (uint32_t)e->model.pass_num;
+  c.qs = e->model.method != PBSIM_METHOD_ERRHMM;  // sample reads use the qshmm event stream
+  c.sample = e->model.method == PBSIM_METHOD_SAMPLE;
+  c.cta_threads = c.qs ? kSimThreads : kErrThreads;
+  c.Pl = {e->d_pool_q.as<uint8_t>(), e->d_pool_start.as<uint64_t>(),
+          (uint32_t)(e->pool_start.empty() ? 0 : e->pool_start.size() - 1)};
+  if (c.sample && !sb) return fail(e, PBSIM_E_INVALID, "internal: sample batch without groups");
+  c.sb = sb;
+  c.spec = c.sample && e->sample_spec && e->sample_spec_run;
+  c.replay = e->run.rng_mode == PBSIM_RNG_REPLAY;
+  c.clip_room = clip_room;
+  int rc = carve_batch(e, n_reads);
+  if (rc) return rc;
+  e->B.first_read = (uint64_t)e->next_read;
+  CK(e->d_ctrl.ensure(64 * 8));
+  CK(e->h_ctrl.ensure(64 * 8));
+  const unsigned long long *hctrl = host_ctrl(e);
+  SimArgs &A = c.A;  // what stays the same over the attempts
+  A.bias_one = e->d_biasone.as<uint8_t>();
+  A.plan_draws = e->strategy == PBSIM_STRATEGY_TRANS ? 3u : (e->strategy == PBSIM_STRATEGY_TEMPL ? 1u : 0u);
+  A.keys.init(e->run.seed, (uint32_t)e->seq_num);
+  A.M = device_model(e);
+  A.G = device_genome(e);
+  A.rng.mode = (uint32_t)e->run.rng_mode;
+  A.rng.seed = e->run.seed;  // the draw log of replay: upload_replay_window
+  A.B = e->B;
+  if (c.replay && (rc = upload_replay_window(e, c))) return rc;
+
+  // (the single, quota-clipped read of a tail batch is segmented too: on one thread a 50 kb read takes milliseconds)
+  // (--method sample: the speculative pass of PHILOX runs; the chains that have to be redone stay sequential)
+  c.use_segments = !c.replay && e->seg_enabled && (!c.sample || c.spec);
+  int seg_retries = 0;
+  for (int attempt = 0; attempt < 9; ++attempt) {
+    if ((rc = plan(e, c))) return rc;
+    if ((rc = size_slots(e, c))) return rc;
+    CK(cudaEventRecord(e->ev_k[0], e->st));
+    pass1_sequential(e, c);
+    if (c.n_seg_total > 0 && (rc = pass1_segments(e, c))) return rc;
+    if (c.spec && (rc = sample_redo(e, c))) return rc;
+    CK(cudaEventRecord(e->ev_k[1], e->st));
+    CK(cudaGetLastError());
+    if ((rc = quota_cut(e, c, attempt))) return rc;
+    const uint32_t flags = (uint32_t)hctrl[2];
+    if (flags & 4u) {
+      // A segmented read could not be completed.  If the only reason is that its window outlasted the segments
+      // provisioned for it (a read that stays in an insertion-rich state of a sticky chain), provision more — the
+      // headroom stays for the batches to come; anything else redoes the batch on the sequential path.
+      const uint32_t inner = flags >> 8;
+      if (inner == 4u && e->seg_extra < 0.6f && seg_retries < 3) {
+        e->seg_extra += 0.04f;
+        ++seg_retries;
+        continue;
+      }
+      c.use_segments = false;
+      e->seg_fallback_batches++;
+      if (attempt >= 8) return fail(e, PBSIM_E_OVERFLOW, "segment-parallel pass 1 failed repeatedly");
+      continue;
+    }
+    if (flags & 1u) {  // a read outgrew its slot: enlarge and redo the batch
+      e->cap_num *= 2;
+      if (attempt >= 8) return fail(e, PBSIM_E_OVERFLOW, "event slots overflowed repeatedly");
+      continue;
+    }
+    const uint64_t cut = hctrl[0];
+    out->cut = cut < n_reads;
+    out->n_valid_reads = out->cut ? (uint32_t)cut : n_reads;
+    out->bases_pass0 = hctrl[1];
+    if (c.replay && hctrl[3] != 0)
+      return fail(e, PBSIM_E_REPLAY, "replay: %llu subreads consumed a different number of draws than the log says",
+                  (unsigned long long)hctrl[3]);
+    break;
+  }
+  return emit_batch(e, c, out);
+}
+
 // ---------------------------------------------------------------------------------------------
 // batch production (the quota loop of pbsim.cpp:2173 / :3792 in batches) and delivery
 // ---------------------------------------------------------------------------------------------
+
+// k_gz_encode's dynamic shared memory: above the 48 KB a launch gets without asking (set in pbsim_cuda_create)
+constexpr size_t kGzEncodeSmem = (size_t)kGzImgWords * 4 + kGzCodes * 256 * 4;
 
 // gzip one record stream of the batch in HBM (gz_kernels.cuh): histogram -> code (host) -> member sizes -> offsets
 // -> members.  Replaces the reference's popen("gzip > file") children (pbsim.cpp:708-730).
@@ -1119,25 +1139,17 @@ int gz_compress(pbsim_engine *e, const uint8_t *in, uint64_t n, DevBuf &dst, uin
   k_gz_size<<<(uint32_t)units, kGzThreads, 0, e->st>>>(in, n, e->d_gz_tables.as<GzTables>(), bgzf ? 1u : 0u,
                                                      e->d_gz_usize.as<uint32_t>(), e->d_gz_ucrc.as<uint32_t>(),
                                                      e->d_gz_usel.as<uint16_t>(), e->d_gz_sbits.as<uint16_t>());
-  k_widen<<<nblk(units, 256), 256, 0, e->st>>>(e->d_gz_usize.as<uint32_t>(), (uint32_t)units, wide);
   CK(cudaMemsetAsync(wide + units, 0, 8, e->st));
-  e->launches += 2;
-  int rc = excl_scan(e, wide, uoff, (uint32_t)units + 1u);
+  e->launches++;
+  const int rc = widen_scan(e, e->d_gz_usize.as<uint32_t>(), (uint32_t)units, wide, uoff);
   if (rc) return rc;
   if (peek(e, hh, uoff + units, 8)) return PBSIM_E_CUDA;
   CK(cudaStreamSynchronize(e->st));
   const uint64_t total = hh[0];
   CK(dst.ensure((size_t)total + 256));
-  static bool attr_set = false;
-  const size_t smem = (size_t)kGzImgWords * 4 + kGzCodes * 256 * 4;
-  if (!attr_set) {
-    CK(cudaFuncSetAttribute(k_gz_encode, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set = true;
-  }
-  k_gz_encode<<<(uint32_t)units, kGzThreads, smem, e->st>>>(in, n, e->d_gz_tables.as<GzTables>(),
-                                                           reinterpret_cast<const uint64_t *>(uoff),
-                                                           e->d_gz_ucrc.as<uint32_t>(), e->d_gz_usel.as<uint16_t>(),
-                                                           e->d_gz_sbits.as<uint16_t>(), bgzf ? 1u : 0u, dst.as<uint8_t>());
+  k_gz_encode<<<(uint32_t)units, kGzThreads, kGzEncodeSmem, e->st>>>(
+      in, n, e->d_gz_tables.as<GzTables>(), reinterpret_cast<const uint64_t *>(uoff), e->d_gz_ucrc.as<uint32_t>(),
+      e->d_gz_usel.as<uint16_t>(), e->d_gz_sbits.as<uint16_t>(), bgzf ? 1u : 0u, dst.as<uint8_t>());
   e->launches++;
   CK(cudaGetLastError());
   *out_bytes = total;
@@ -1554,6 +1566,14 @@ int pbsim_cuda_create(pbsim_engine **out, int device) {
                 ce == cudaSuccess ? "device count is 0" : cudaGetErrorString(ce));
   if (device < 0 || device >= n) return fail(e, PBSIM_E_INVALID, "device %d out of range (0..%d)", device, n - 1);
   CK(cudaSetDevice(device));
+  // Function attributes belong to the function as loaded on one device, so every engine sets them on its own.
+  // k_emit_rows' staging rows need shared memory for 4 CTAs per SM; k_chain_chunk gets the largest carve-out too.
+  CK(cudaFuncSetAttribute(k_chain_chunk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_QSHMM>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                          cudaSharedmemCarveoutMaxShared));
+  CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_ERRHMM>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                          cudaSharedmemCarveoutMaxShared));
+  CK(cudaFuncSetAttribute(k_gz_encode, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGzEncodeSmem));
   pbsim_engine *ne = new pbsim_engine();
   ne->device = device;
   cudaError_t c1 = cudaStreamCreateWithFlags(&ne->st, cudaStreamNonBlocking);
@@ -1582,32 +1602,17 @@ void pbsim_cuda_destroy(pbsim_engine *e) {
   stop_producer(e);
   cudaStreamSynchronize(e->st_copy);
   cudaStreamSynchronize(e->st);
-  DevBuf *bufs[] = {&e->d_blob, &e->d_acc, &e->d_prob2len, &e->d_prob2acc, &e->d_qs_tabs, &e->d_qs_thr_hp, &e->d_qs_thr_hp32,
-                    &e->d_er_bias, &e->d_ascii, &e->d_pk, &e->d_hp4, &e->d_xm, &e->d_hpfreq, &e->d_biasone, &e->d_flag,
-                    &e->d_draws, &e->d_starts, &e->b_read_u32, &e->b_sub_u32, &e->b_sub_u64, &e->b_sub_f64, &e->d_bins,
-                    &e->d_ctrl, &e->d_cub_tmp, &e->d_ev, &e->d_ck, &e->out[0].reads, &e->out[0].maf, &e->out[1].reads, &e->out[1].maf, &e->d_stats, &e->d_seg,
-                    &e->d_seg_bins, &e->d_set_start, &e->d_set_rprefix, &e->d_set_plus, &e->d_set_ids, &e->d_set_idstart,
-                    &e->d_set_ssp_ends, &e->d_set_ssp_mod, &e->d_set_first, &e->d_map_tr, &e->d_map_k, &e->gz[0].reads, &e->gz[0].maf, &e->gz[1].reads,
-                    &e->gz[1].maf, &e->d_gz_tables, &e->d_gz_hist, &e->d_gz_usize, &e->d_gz_ucrc, &e->d_gz_uoff, &e->d_gz_usel, &e->d_gz_sbits,
-                    &e->d_lay, &e->d_tile_sub, &e->d_tile_desc, &e->d_chunk, &e->d_chunk_bins};
-  for (DevBuf *b : bufs) b->release();
-  for (auto &a : e->h_stage)
-    for (auto &b : a) b.release();
   cudaEventDestroy(e->ev_copy);
   for (auto &ev : e->ev_k) cudaEventDestroy(ev);
   for (auto &ev : e->ev_user) cudaEventDestroy(ev);
   for (auto &ev : e->ev_gz) cudaEventDestroy(ev);
   for (auto &ev : e->ev_seg) cudaEventDestroy(ev);
   for (auto &ev : e->ev_chain) cudaEventDestroy(ev);
-  e->h_gz.release();
-  e->h_ctrl.release();
-  e->h_acc.release();
-  e->h_stats.release();
   cudaEventDestroy(e->ev0);
   cudaEventDestroy(e->ev1);
   cudaStreamDestroy(e->st);
   cudaStreamDestroy(e->st_copy);
-  delete e;
+  delete e;  // the buffers free themselves, on the engine's device
 }
 
 int pbsim_cuda_set_model(pbsim_engine *e, const pbsim_model *m) {
@@ -1711,10 +1716,8 @@ int pbsim_cuda_set_sequence(pbsim_engine *e, const pbsim_sequence *s) {
   if (!e || !s || !s->bases) return PBSIM_E_INVALID;
   CK(cudaSetDevice(e->device));
   if (s->len < 1 || s->len > 1000000000) return fail(e, PBSIM_E_INVALID, "sequence length out of range");
-  const size_t padded = ((size_t)s->len + 15) / 16 * 16 + 64;
-  CK(e->d_ascii.ensure(padded));
-  CK(cudaMemsetAsync(e->d_ascii.as<uint8_t>() + (s->len / 16) * 16, 0, padded - (s->len / 16) * 16, e->st));
-  CK(cudaMemcpyAsync(e->d_ascii.p, s->bases, (size_t)s->len, cudaMemcpyHostToDevice, e->st));
+  const int rc = upload_ascii(e, s->bases, s->len);
+  if (rc) return rc;
   e->strategy = PBSIM_STRATEGY_WGS;
   return finish_sequence_ingest(e, s->len, s->seq_num, s->hp_del_bias);
 }
@@ -1791,10 +1794,7 @@ int pbsim_cuda_set_seqset(pbsim_engine *e, const pbsim_seqset *s) {
     if ((rc = upload(e, e->d_set_ssp_mod, mod.data(), mod.size()))) return rc;
     CK(cudaStreamSynchronize(e->st));  // the vectors go out of scope
   }
-  const size_t padded = ((size_t)total + 15) / 16 * 16 + 64;
-  CK(e->d_ascii.ensure(padded));
-  CK(cudaMemsetAsync(e->d_ascii.as<uint8_t>() + (total / 16) * 16, 0, padded - (total / 16) * 16, e->st));
-  CK(cudaMemcpyAsync(e->d_ascii.p, s->bases, (size_t)total, cudaMemcpyHostToDevice, e->st));
+  if ((rc = upload_ascii(e, s->bases, total))) return rc;
   // only simulate_by_qshmm_trans upper-cases the first base (:2774; :3330, :4474, :5049 start at 1)
   const bool keep_first = !(trans && e->model.method == PBSIM_METHOD_QSHMM);
   rc = finish_sequence_ingest(e, total, 0, s->hp_del_bias, keep_first);
@@ -1805,9 +1805,8 @@ int pbsim_cuda_set_synthetic_sequence(pbsim_engine *e, int64_t len, int32_t seq_
   if (!e) return PBSIM_E_INVALID;
   CK(cudaSetDevice(e->device));
   if (len < 1 || len > 1000000000) return fail(e, PBSIM_E_INVALID, "sequence length out of range");
-  const size_t padded = ((size_t)len + 15) / 16 * 16 + 64;
-  CK(e->d_ascii.ensure(padded));
-  CK(cudaMemsetAsync(e->d_ascii.as<uint8_t>() + (len / 16) * 16, 0, padded - (len / 16) * 16, e->st));
+  const int rc = upload_ascii(e, nullptr, len);
+  if (rc) return rc;
   k_synth_ascii<<<nblk((len + 15) / 16, 256), 256, 0, e->st>>>(e->d_ascii.as<uint8_t>(), len, seed);
   e->launches++;
   double bias[12] = {0, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0};
