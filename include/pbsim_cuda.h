@@ -172,7 +172,7 @@ typedef struct {
   double deflate_seconds;        /* ... of which the gzip writer (option "deflate")          */
   double seg_seconds;            /* ... of which the segment kernel (k_sim_seg / _err) alone  */
   int64_t kernel_launches;       /* number of engine kernels launched during the run         */
-  double chain_seconds;          /* ... of which the chain / quality kernel (k_chain_chunk / _err) alone (ABI 4) */
+  double chain_seconds;          /* ... of which the chain-chunk kernel (k_qs_pass1 / k_chain_chunk_err) alone (ABI 4) */
   int64_t len_total_end;         /* the quota counter when the run ended: len_total_start + the bases this run's *
                                   * reads emitted in pass 0 (:2297) = len_total_start of the next read range (ABI 4) */
 } pbsim_stats;

@@ -740,8 +740,9 @@ void pass1_sequential(pbsim_engine *e, BatchCtx &c) {
   e->launches++;
 }
 
-// segment-parallel pass 1 for the long reads (seg_kernels.cuh): the chain-only pass computes the HMM state in front of
-// every segment (k_chain_chunk), then the segments run and k_find_end finds where each read ends
+// segment-parallel pass 1 for the long reads (seg_kernels.cuh): chain chunks recover the HMM state in front of their
+// segments (qshmm model accuracies: and simulate them, k_qs_pass1), the other segments run (k_sim_seg, k_sim_seg_err)
+// and k_find_end finds where each read ends
 int pass1_segments(pbsim_engine *e, BatchCtx &c) {
   const Batch &B = e->B;
   const uint32_t nseg = (uint32_t)c.n_seg_total;
@@ -752,11 +753,17 @@ int pass1_segments(pbsim_engine *e, BatchCtx &c) {
   uint32_t *u = reinterpret_cast<uint32_t *>(S.seg_res + nseg);
   uint32_t **seg_arrays[] = {&S.seg_sub, &S.seg_key_in, &S.seg_key_out, &S.seg_id_in, &S.seg_order, &S.seg_state};
   for (size_t i = 0; i < 6; ++i) *seg_arrays[i] = u + i * nseg;
-  k_seg_fill<<<nblk(B.n_sub, 256), 256, 0, e->st>>>(B, S, c.pass);
-  CtaSchedule sc;
-  int rc = schedule_ctas(e, e->d_seg_bins, S.seg_key_in, S.seg_key_out, S.seg_id_in, S.seg_order, nseg, 20, c.cta_threads,
-                         false, &sc);
-  if (rc) return rc;
+  // qshmm: k_qs_pass1 simulates the segments of model accuracies, k_sim_seg the others (if the model has accuracies
+  // without a chain) and those of --method sample
+  bool freq_only = false;
+  for (const AccEntry &a : e->img.acc) freq_only |= a.valid && !a.has_model;
+  const bool seg_pass = !c.qs || c.sample || freq_only;
+  k_seg_fill<<<nblk(B.n_sub, 256), 256, 0, e->st>>>(B, S, c.pass, c.qs && !c.sample ? 1u : 0u);
+  CtaSchedule sc = {};
+  int rc = 0;
+  if (seg_pass && (rc = schedule_ctas(e, e->d_seg_bins, S.seg_key_in, S.seg_key_out, S.seg_id_in, S.seg_order, nseg, 20,
+                                      c.cta_threads, false, &sc)))
+    return rc;
   SegArgs SA;
   SA.keys = c.A.keys;
   SA.M = c.A.M;
@@ -786,7 +793,7 @@ int pass1_segments(pbsim_engine *e, BatchCtx &c) {
     SegArgs CA = SA;
     set_ctas(CA, cc);
     CK(cudaEventRecord(e->ev_chain[0], e->st));
-    if (c.qs) k_chain_chunk<<<cc.slots, kChainThreads, kQsSmemBytes, e->st>>>(CA, C);
+    if (c.qs) k_qs_pass1<<<cc.slots, kChainThreads, kQsSmemBytes, e->st>>>(CA, C);
     else k_chain_chunk_err<<<cc.slots, kErrThreads, e->er_smem_bar_off + 16, e->st>>>(CA, C, e->er_smem_bar_off);
     CK(cudaEventRecord(e->ev_chain[1], e->st));
     e->launches += 2;
@@ -795,7 +802,8 @@ int pass1_segments(pbsim_engine *e, BatchCtx &c) {
   const uint32_t end_grid = nblk((uint64_t)B.n_sub * 32, 128);
   if (c.qs) {
     if (c.sample) k_sim_seg<true><<<sc.slots, kSimThreads, 0, e->st>>>(SA);
-    else k_sim_seg<false><<<sc.slots, kSimThreads, 0, e->st>>>(SA);
+    else if (seg_pass) k_sim_seg<false><<<sc.slots, kSimThreads, 0, e->st>>>(SA);
+    e->launches += seg_pass ? 1 : 0;
     CK(cudaEventRecord(e->ev_seg[1], e->st));
     k_find_end<<<end_grid, 128, 0, e->st>>>(B, S, c.A.G, SA.bias_one, c.pass, SA.ev, e->d_ck.as<Ckpt>(), c.A.M.qs_fast,
                                             c.sample ? 1u : 0u);
@@ -803,8 +811,9 @@ int pass1_segments(pbsim_engine *e, BatchCtx &c) {
     k_sim_seg_err<<<sc.slots, kErrThreads, e->er_smem_bar_off + 16, e->st>>>(SA, e->er_smem_bar_off);
     CK(cudaEventRecord(e->ev_seg[1], e->st));
     k_find_end_err<<<end_grid, 128, 0, e->st>>>(B, S, c.A.G, SA.keys, SA.bias_one, c.pass, SA.ev, e->d_ck.as<Ckpt>());
+    e->launches++;
   }
-  e->launches += 3;
+  e->launches += 2;
   e->seg_batches++;
   return 0;
 }
@@ -1567,8 +1576,8 @@ int pbsim_cuda_create(pbsim_engine **out, int device) {
   if (device < 0 || device >= n) return fail(e, PBSIM_E_INVALID, "device %d out of range (0..%d)", device, n - 1);
   CK(cudaSetDevice(device));
   // Function attributes belong to the function as loaded on one device, so every engine sets them on its own.
-  // k_emit_rows' staging rows need shared memory for 4 CTAs per SM; k_chain_chunk gets the largest carve-out too.
-  CK(cudaFuncSetAttribute(k_chain_chunk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  // k_emit_rows' staging rows need shared memory for 4 CTAs per SM; k_qs_pass1 gets the largest carve-out too.
+  CK(cudaFuncSetAttribute(k_qs_pass1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_QSHMM>, cudaFuncAttributePreferredSharedMemoryCarveout,
                           cudaSharedmemCarveoutMaxShared));
   CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_ERRHMM>, cudaFuncAttributePreferredSharedMemoryCarveout,

@@ -4,10 +4,11 @@
 // units are the same size whatever the read lengths are (1 kb or 1 Mb), which removes the sequential critical
 // path a whole-read-per-thread schedule has.  qshmm splits the work by what is sequential and what is not:
 //   k_seg_fill    : (sub-read, k) list of all segments of the batch + accuracy sort key
-//   k_chain_chunk : QUALITY pass.  One thread per chunk of segments: exact entry state by backward coupling, then
-//                   the HMM chain + emission walk; writes the quality value of every position into its event slot
-//   k_sim_seg     : ERROR pass.  One WARP per segment, consecutive lanes on consecutive positions: error draw,
-//                   choices, deletion run of every position -> the event, in place over the quality (coalesced)
+//   k_qs_pass1    : model accuracies.  One thread per chunk of segments: exact entry state by backward coupling,
+//                   then the HMM chain + emission walk and, position by position, the error draw, choices and
+//                   deletion run -> the events and the segments' totals
+//   k_sim_seg     : accuracies without a model (and --method sample).  One WARP per segment, consecutive lanes on
+//                   consecutive positions: quality, error draw, choices, deletion run -> the event (coalesced)
 //   k_find_end    : one warp per segmented sub-read: prefix over its segments, deletion-run repairs, clip at the
 //                   window end, tile checkpoints, totals
 #pragma once
@@ -27,20 +28,22 @@ struct SegBatch {
   uint32_t *seg_id_in;
   uint32_t *seg_order;       // segments sorted by accuracy
   SegResult *seg_res;        // [n_seg_total] indexed by segment id
-  uint32_t *seg_state;       // [n_seg_total] chain state in front of a segment (recorded by k_chain_chunk)
+  uint32_t *seg_state;       // [n_seg_total] chain state in front of a segment (recorded by k_chain_chunk_err)
 };
 
-// thread per sub-read: write its segments' descriptors
-__global__ void k_seg_fill(Batch B, SegBatch S, uint32_t pass_num) {
+// thread per sub-read: write its segments' descriptors.  skip_chained: the segments of reads whose chain chunks
+// simulate them (qshmm model accuracies, k_qs_pass1) get the out-of-range bin kBins, so k_sim_seg skips them
+__global__ void k_seg_fill(Batch B, SegBatch S, uint32_t pass_num, uint32_t skip_chained) {
   const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= B.n_sub) return;
   const uint64_t lo = S.seg_off[s], hi = S.seg_off[s + 1];
   if (hi == lo) return;
   const uint32_t meta = B.plan_meta[s / pass_num];
   const uint32_t acc = meta & 0xFFu;
+  const bool skip = skip_chained != 0u && B.nchunk[s] != 0u;
   for (uint64_t i = lo; i < hi; ++i) {
     S.seg_sub[i] = s;
-    S.seg_key_in[i] = acc << 21;
+    S.seg_key_in[i] = skip ? ((uint32_t)kBins << 20) : acc << 21;
     S.seg_id_in[i] = (uint32_t)i;
   }
 }
@@ -48,7 +51,7 @@ __global__ void k_seg_fill(Batch B, SegBatch S, uint32_t pass_num) {
 // ---- chain chunks: the threads that recover the HMM state in front of every segment -------------------------------
 struct ChunkBatch {
   uint32_t n_chunks, per_chunk;   // per_chunk: segments walked by one chunk (reads of sticky chains: all of them)
-  uint32_t qs;                    // 1: qshmm (the quality pass walks every segment)
+  uint32_t qs;                    // 1: qshmm (k_qs_pass1 walks every segment)
   const uint64_t *chunk_off;      // [n_sub + 1] exclusive scan of Batch::nchunk
   uint32_t *sub, *key_in, *key_out, *id_in, *order;
 };
@@ -64,7 +67,7 @@ __global__ void k_chunk_fill(Batch B, ChunkBatch C, uint32_t pass_num) {
   for (uint64_t i = lo; i < hi; ++i) {
     // longest walk first inside an accuracy (the same key layout as the sequential schedule)
     // errhmm records the state in front of segments k_from+1 .. k_to (nobody needs the one behind the last
-    // segment); the qshmm quality pass walks every segment
+    // segment); qshmm's k_qs_pass1 walks every segment
     const bool qs = C.qs != 0u;
     const uint32_t k_from = (uint32_t)(i - lo) * per, k_to = min(k_from + per, qs ? nseg : nseg - 1u);
     const uint32_t work = k_to - k_from + (k_from > 0u ? 1u : 0u);
@@ -88,15 +91,16 @@ struct SegArgs {
   const uint64_t *pool_start;
 };
 
-// ERROR pass of the qshmm segments: one WARP per segment, lane l of iteration i on positions 128 i + 4 l .. + 3.
-// The slot holds the qualities the quality pass wrote (accuracies without a model: computed here from the freq2qc
-// table); events replace them in place with 8-byte loads and stores, consecutive lanes on consecutive addresses.
+// The qshmm segments without chain chunks (accuracies without a model, --method sample): one WARP per segment, lane l
+// of iteration i on positions 128 i + 4 l .. + 3.  The qualities come from the freq2qc table or the pool entry; the
+// events are written with 8-byte stores, consecutive lanes on consecutive addresses.
 // A CTA serves kSimThreads segments of one accuracy (the schedule of the other pass-1 kernels), warp w the
 // segments lo + w, lo + w + 4, ...
 constexpr int kSegWarps = kSimThreads / 32;
-// threads of a quality-pass CTA (they share one accuracy's tables, 28 KB: 8 CTAs per SM with the largest shared-memory
-// carve-out).  Measured: 256-thread CTAs (48 warps per SM) are 15 % slower on the pass (c3 and c1, chunks of 8
-// segments), 512-thread CTAs likewise with chunks of 32 — more warps only queue up behind the shared-memory pipe.
+// threads of a chain-chunk CTA (they share one accuracy's tables, 30 KB: 7 CTAs per SM with the largest shared-memory
+// carve-out).  Measured on the quality pass alone: 256-thread CTAs (48 warps per SM) were 15 % slower (c3 and c1,
+// chunks of 8 segments), 512-thread CTAs likewise with chunks of 32 — more warps only queue up behind the shared-memory
+// pipe.
 #ifndef PB_CHAIN_THREADS
 #define PB_CHAIN_THREADS 128
 #endif
@@ -162,16 +166,12 @@ __global__ void __launch_bounds__(kSimThreads) k_sim_seg(SegArgs A) {
         for (uint32_t u = 0; u < PB_GROUP; ++u) b[u] = p + u < len ? (uint32_t)__ldg(qp + p + u) - 33u : 0u;
         q[it] = make_uint2(b[0] | (b[1] << 16), b[2] | (b[3] << 16));
       }
-    } else if (ae.has_model) {
-#pragma unroll
-      for (uint32_t it = 0; it < kIters; ++it)
-        q[it] = *reinterpret_cast<const uint2 *>(ev + lane * PB_GROUP + it * 32u * PB_GROUP);
     }
 #pragma unroll
     for (uint32_t it = 0; it < kIters; ++it) {
       const uint32_t j = lane * PB_GROUP + it * 32u * PB_GROUP;
       uint32_t qv[PB_GROUP];
-      if (SAMPLE || ae.has_model) {
+      if (SAMPLE) {
         qv[0] = q[it].x & 0x7Fu; qv[1] = (q[it].x >> 16) & 0x7Fu; qv[2] = q[it].y & 0x7Fu; qv[3] = (q[it].y >> 16) & 0x7Fu;
       } else {
         qs_freq_qualities(T, A.keys, read_id, c1, k * PB_TILE + j, qv);
@@ -215,10 +215,10 @@ __global__ void __launch_bounds__(kSimThreads) k_sim_seg(SegArgs A) {
   }
 }
 
-// QUALITY pass (qshmm): one thread per chain chunk.  Exact state at the chunk's first position by backward
-// coupling (init draw at position 0), then the chain + emission walk through the chunk's segments, which writes
-// the quality of every position into its event slot (qshmm_quality_range); k_sim_seg turns them into events.
-__global__ void __launch_bounds__(kChainThreads) k_chain_chunk(SegArgs A, ChunkBatch C) {
+// PASS 1 of the qshmm segments of model accuracies: one thread per chain chunk.  Exact state at the chunk's first
+// position by backward coupling (init draw at position 0), then qualities and events of every position of the
+// chunk's segments in one walk (qshmm_chunk_pass1), which also writes the segments' SegResults.
+__global__ void __launch_bounds__(kChainThreads) k_qs_pass1(SegArgs A, ChunkBatch C) {
   extern __shared__ __align__(128) uint8_t smem[];
   uint32_t acc, lo, hi;
   if (!cta_assignment(A.cta_order, A.cta_first, A.bin_lo, A.bin_hi, &acc, &lo, &hi)) return;
@@ -227,8 +227,9 @@ __global__ void __launch_bounds__(kChainThreads) k_chain_chunk(SegArgs A, ChunkB
   if (threadIdx.x == 0) mbar_init(bar, 1);
   __syncthreads();
   if (threadIdx.x == 0) {
-    mbar_expect_tx(bar, ae.blob_bytes);
+    mbar_expect_tx(bar, ae.blob_bytes + PBSIM_NQV * 16u);
     tma_bulk_g2s(smem, A.M.blob + ae.blob_off, ae.blob_bytes, bar);
+    tma_bulk_g2s(smem + kQsSmemFast, A.M.qs_fast, PBSIM_NQV * 16u, bar);
   }
   mbar_wait(bar, 0);
   const uint32_t i = lo + threadIdx.x;
@@ -252,9 +253,9 @@ __global__ void __launch_bounds__(kChainThreads) k_chain_chunk(SegArgs A, ChunkB
   T.thr = nullptr;
   T.thr_hp = nullptr;
   T.qc_prob = nullptr;
-  T.thr32 = nullptr;
+  T.thr32 = reinterpret_cast<const QsThr *>(A.M.qs_thr32);  // global: only the rare hp[-1] rule reads it
   T.thr_hp32 = nullptr;
-  T.fast = nullptr;
+  T.fast = reinterpret_cast<const QsFast *>(smem + kQsSmemFast);
   uint32_t row = 0, mod = ae.init_mod, emod = 1;
   if (k_from > 0u) {
     QsSegAux X;
@@ -265,8 +266,8 @@ __global__ void __launch_bounds__(kChainThreads) k_chain_chunk(SegArgs A, ChunkB
   }
   // the coupling loops leave the lanes of a warp at different points: reconverge before the walk
   __syncwarp();
-  qshmm_quality_range(T, A.keys, read_id, pass, row, mod, emod, k_from, k_to,
-                      reinterpret_cast<uint16_t *>(A.ev) + A.B.ev_off[s]);
+  qshmm_chunk_pass1(T, A.keys, read_id, pass, row, mod, k_from, k_to, reinterpret_cast<uint16_t *>(A.ev) + A.B.ev_off[s],
+                    A.S.seg_res + A.S.seg_off[s]);
 }
 
 // the same for errhmm: chunk 0 walks from column 0 (the init row is drawn until a read base exists, :3853)

@@ -838,15 +838,17 @@ PB_HD void qshmm_simulate_fast(const QsView &T, const PhiloxKeys &K, uint32_t re
 // ---------------------------------------------------------------------------------------------
 // qshmm SEGMENT-PARALLEL pass 1 (PHILOX, reads that never need the genome in pass 1).
 // A read is cut into segments of PB_TILE read positions; the work is split by what is sequential and what is not:
-//   * the QUALITY pass (k_chain_chunk): the HMM chain is the only sequential part of a read.  One thread walks a
-//     chunk of segments through the chain (its own Philox stream, one block per 4 positions) and writes the
-//     QUALITY VALUE of every position into the segment's event slot.  The state entering a chunk is recovered
-//     EXACTLY by backward coupling: run every reachable state through the positions just before the chunk with
-//     those positions' own draws; as soon as all images coincide the state is independent of the earlier history
-//     (if the window reaches position 0 the init draw decides).
-//   * the ERROR pass (k_sim_seg): given its quality, a position depends on nothing but its own two error-stream
-//     words, so one WARP handles a segment with consecutive lanes on consecutive positions (coalesced loads and
-//     stores, no divergence): error draw, choices, deletion run -> the event, written over the quality in place.
+//   * the QUALITY pass: the HMM chain is the only sequential part of a read.  One thread walks a chunk of segments
+//     through the chain (its own Philox stream, one block per 4 positions).  The state entering a chunk is
+//     recovered EXACTLY by backward coupling: run every reachable state through the positions just before the
+//     chunk with those positions' own draws; as soon as all images coincide the state is independent of the
+//     earlier history (if the window reaches position 0 the init draw decides).
+//   * the ERROR pass: given its quality, a position depends on nothing but its own two error-stream words: error
+//     draw, choices, deletion run -> the event.
+//   Model accuracies run both in the same thread (k_qs_pass1, qshmm_chunk_pass1): the chain's lookups leave issue
+//   slots free that the error pass's arithmetic fills, and a quality never travels through memory.  Accuracies
+//   without a model have no chain: one WARP handles a segment (k_sim_seg), consecutive lanes on consecutive
+//   positions, qualities from the freq2qc table.
 // Segments are simulated "unbounded" (they cannot know the reference offset they start at); find_end then locates
 // the position at which the window is used up, clips the last deletion run and drops the rest, which is what the
 // sequential loop `while (ref_offset < mut.len)` (:2213, :2268) does.
@@ -927,10 +929,10 @@ PB_HD void store_u16x8(uint16_t *dst, const uint32_t v[4]) {  // dst is 16-byte 
 #endif
 }
 
-// QUALITY pass over segments k_from .. k_to-1 of a read from the state (row, mod, emod) that enters segment k_from:
-// the quality value of every position goes into bits 0-6 of its entry in the segment's slot (uint16 per position,
-// 8 positions per 16-byte store).  The lookups form one dependent chain (table entry -> next row); the Philox
-// blocks of the NEXT eight positions do not depend on it and are computed alongside.
+// QUALITY pass alone over segments k_from .. k_to-1 of a read from the state (row, mod, emod) that enters segment
+// k_from: the quality value of every position goes into bits 0-6 of its entry in the segment's slot, for
+// qshmm_error_segment to turn into events.  The kernels run both passes in one walk (qshmm_chunk_pass1); this split
+// statement is what the CPU harness runs, and the reference the fused walk is tested against.
 PB_HD void qshmm_quality_range(const QsView &T, const PhiloxKeys &K, uint32_t read_id, uint32_t pass, uint32_t row,
                                uint32_t mod, uint32_t emod, uint32_t k_from, uint32_t k_to, uint16_t *slots) {
   const uint32_t c1 = pass << 16;
@@ -987,10 +989,10 @@ PB_HD uint32_t pb_popc(uint32_t x) {
   return (uint32_t)__builtin_popcount(x);
 #endif
 }
-PB_HD void qs_error_lane(const QsFast *fast, const PhiloxKeys &K, uint32_t read_id, uint32_t c1, uint32_t p,
-                         const uint32_t qv[PB_GROUP], uint32_t &w0, uint32_t &w1, QsLaneTotals &t) {
-  uint32_t x[PB_GROUP], y[PB_GROUP], e[PB_GROUP];
-  error_words(K, read_id, c1, p, x, y);
+// qs_error_group: the same from the positions' error-stream words (error_words) given; qs_error_lane computes them
+PB_HD void qs_error_group(const QsFast *fast, const uint32_t qv[PB_GROUP], const uint32_t x[PB_GROUP],
+                          const uint32_t y[PB_GROUP], uint32_t &w0, uint32_t &w1, QsLaneTotals &t) {
+  uint32_t e[PB_GROUP];
 #pragma unroll
   for (uint32_t u = 0; u < PB_GROUP; ++u) {
     const QsFast th = fast[qv[u]];
@@ -1006,6 +1008,12 @@ PB_HD void qs_error_lane(const QsFast *fast, const PhiloxKeys &K, uint32_t read_
   t.nins += pb_popc((w0 & 0x01000100u) | ((w1 & 0x01000100u) << 1));
   const uint32_t dd = ((w0 >> 12) & 0x000F000Fu) + ((w1 >> 12) & 0x000F000Fu);
   t.ndel += (dd & 0xFFFFu) + (dd >> 16);
+}
+PB_HD void qs_error_lane(const QsFast *fast, const PhiloxKeys &K, uint32_t read_id, uint32_t c1, uint32_t p,
+                         const uint32_t qv[PB_GROUP], uint32_t &w0, uint32_t &w1, QsLaneTotals &t) {
+  uint32_t x[PB_GROUP], y[PB_GROUP];
+  error_words(K, read_id, c1, p, x, y);
+  qs_error_group(fast, qv, x, y, w0, w1, t);
 }
 
 // ERROR pass, first segment of a read: while the reference offset is still 0 (leading insertions) the deletion
@@ -1094,7 +1102,8 @@ PB_HD void qshmm_segment_generic(const QsView &T, const PhiloxKeys &K, uint32_t 
 }
 
 // ERROR pass over one segment, as the warp of k_sim_seg runs it (sequential statement for the CPU harness: the
-// 256 lane steps one after the other).  The slot holds the qualities on entry (model accuracies).
+// 256 lane steps one after the other).  With T.has_model the slot holds the qualities on entry (qshmm_quality_range's,
+// or --method sample: the pool entry's); otherwise they come from the freq2qc table.
 PB_HD void qshmm_error_segment(const QsView &T, const PhiloxKeys &K, uint32_t read_id, uint32_t pass, uint32_t p_start,
                                bool first_segment, uint16_t *ev, SegResult &res) {
   const uint32_t c1 = pass << 16;
@@ -1132,6 +1141,65 @@ PB_HD void qshmm_error_segment(const QsView &T, const PhiloxKeys &K, uint32_t re
   res.flags = 0;
   res.pad = 0;
   res.prob = prob;
+}
+
+// PASS 1 of segments k_from .. k_to-1 of a read of a MODEL accuracy, from the state (row, mod) that enters segment
+// k_from: the quality pass (chain + emission lookups) and the error pass (qs_error_group) of every position in one
+// walk, 8 positions per group, whose events go out with one 16-byte store; the totals of segment k go to res[k].
+// The lookups form one dependent chain (table entry -> next row); the Philox blocks of a group (chain words of the
+// NEXT group, error words of this one) do not depend on it and are computed alongside.  A quality is never stored on
+// its own: a segment with an entry of >= PB_QS_DEL_SAT deletions (rare) takes its qualities back from bits 0-6 of the
+// events it wrote and is redone by qshmm_segment_generic.
+PB_HD void qshmm_chunk_pass1(const QsView &T, const PhiloxKeys &K, uint32_t read_id, uint32_t pass, uint32_t row,
+                             uint32_t mod, uint32_t k_from, uint32_t k_to, uint16_t *slots, SegResult *res) {
+  const uint32_t c1 = pass << 16;
+  uint32_t nx[8];
+  philox_block_keys(K, (k_from * PB_TILE) >> 2, c1, read_id, 2u, nx);
+  philox_block_keys(K, ((k_from * PB_TILE) >> 2) + 1u, c1, read_id, 2u, nx + 4);
+  for (uint32_t k = k_from; k < k_to; ++k) {
+    uint16_t *slot = slots + (uint64_t)k * PB_SEG_STRIDE;
+    QsLaneTotals t;
+    t.nsub = t.nins = t.ndel = t.prob = t.big = 0;
+    uint64_t prob = 0;
+    for (uint32_t j = 0; j < PB_TILE; j += 8u) {
+      const uint32_t p = k * PB_TILE + j;
+      uint32_t cw[8], x[8], y[8], qv[8], w[4];
+#pragma unroll
+      for (uint32_t u = 0; u < 8u; ++u) cw[u] = nx[u];
+      philox_block_keys(K, (p >> 2) + 2u, c1, read_id, 2u, nx);
+      philox_block_keys(K, (p >> 2) + 3u, c1, read_id, 2u, nx + 4);
+      error_words(K, read_id, c1, p, x, y);
+      error_words(K, read_id, c1, p + 4u, x + 4, y + 4);
+#pragma unroll
+      for (uint32_t u = 0; u < 8u; ++u) {
+        const uint32_t e = T.t2[row + mulhi32(cw[u] & 0xFFFF0000u, mod)];
+        row = e & 0xFFFFu;
+        mod = (e >> 16) & 0xFFu;
+        qv[u] = T.emis[row + mulhi32(cw[u] << 16, e >> 24)];
+      }
+      t.prob = 0;  // 8 positions of at most 2^PB_PROB_SHIFT each
+      qs_error_group(T.fast, qv, x, y, w[0], w[1], t);
+      qs_error_group(T.fast, qv + 4, x + 4, y + 4, w[2], w[3], t);
+      prob += t.prob;
+      store_u16x8(slot + j, w);
+    }
+    if (t.big) {
+      uint8_t q[PB_TILE];
+      for (uint32_t j = 0; j < PB_TILE; ++j) q[j] = (uint8_t)(slot[j] & 0x7Fu);
+      qshmm_segment_generic(T, K, read_id, pass, k * PB_TILE, k == 0, q, slot, res[k]);
+      continue;
+    }
+    if (k == 0) t.ndel -= qs_fix_leading(T, K, read_id, c1, slot);
+    SegResult r;
+    r.n_entries = PB_TILE;
+    r.ref_adv = PB_TILE - t.nins + t.ndel;
+    r.nsub = t.nsub;
+    r.ndel = t.ndel;
+    r.flags = 0;
+    r.pad = 0;
+    r.prob = prob;
+    res[k] = r;
+  }
 }
 
 // Reference bases after which no deletion can follow: in the default bias mode hp_del_bias[hp] is 1 for hp 1..10

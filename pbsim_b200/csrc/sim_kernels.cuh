@@ -87,7 +87,7 @@ struct Batch {
   uint64_t *ck_off;
   uint32_t *nent, *rlen, *ncol, *nsub, *nins, *ndel, *flags, *draws_used;
   uint32_t *nseg;          // segments provisioned (0: the sub-read runs on the sequential pass-1 path)
-  uint32_t *nchunk;        // chain chunks: threads of k_chain_chunk that recover the states in front of its segments
+  uint32_t *nchunk;        // chain chunks: threads of k_qs_pass1 / k_chain_chunk_err that walk its segments
   double *accuracy;
   // --method sample, per read: which copy of its group (pool entry, pool pass) a read is, and the group's size
   uint32_t *grp_copy, *grp_num;
@@ -170,9 +170,9 @@ __global__ void k_plan(DeviceModel M, DeviceGenome G, DeviceSet S, RngParams rng
   const bool errm = M.method == PBSIM_METHOD_ERRHMM;
   const bool segmented = seg_min_len != 0u && rng.mode == PBSIM_RNG_PHILOX && (!slow || M.uniform_bias) && ae.valid &&
                          p.wlen >= seg_min_len && !(errm && ae.mode == 3u);
-  // The HMM state in front of every segment comes from a chain-only pass (k_chain_chunk): a thread per CHUNK of
-  // chain_chunk segments starts from the exact state recovered by backward coupling at the chunk's first position
-  // (position 0: the init draw) and walks just the state chain through the chunk.  Chains with sticky states do not
+  // The HMM state in front of every segment comes from chain chunks (k_qs_pass1, k_chain_chunk_err): a thread per
+  // CHUNK of chain_chunk segments starts from the exact state recovered by backward coupling at the chunk's first
+  // position (position 0: the init draw) and walks the chain through the chunk.  Chains with sticky states do not
   // couple quickly: their reads are one chunk.
   const bool needs_chain = segmented && (errm || ae.has_model);
   const uint32_t nseg = segmented ? qshmm_segments_for(p.wlen, ae.rho * (1.0f + seg_extra)) : 0u;
@@ -183,7 +183,7 @@ __global__ void k_plan(DeviceModel M, DeviceGenome G, DeviceSet S, RngParams rng
   if (segmented) cap = (uint64_t)nseg * (errm ? PB_TILE : PB_SEG_STRIDE) + 64u;
   cap = (cap + ev_align - 1u) / ev_align * ev_align;
   const uint32_t ckc = segmented ? nseg + 2u : (uint32_t)(cap / PB_TILE) + 2u;
-  // the quality pass walks EVERY provisioned segment (it writes the quality of every position)
+  // qshmm's k_qs_pass1 walks EVERY provisioned segment (it writes the events of every position)
   uint32_t nchunk = 0;
   if (needs_chain && nseg > 0u) nchunk = ae.seg_ok ? (nseg + chain_chunk - 1u) / chain_chunk : 1u;
   for (uint32_t h = 0; h < M.pass_num; ++h) {
