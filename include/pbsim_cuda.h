@@ -146,7 +146,7 @@ typedef struct {
 typedef struct {
   const char *reads;        /* FASTQ (pass_num == 1) or SAM records (no @HD/@RG header)      */
   int64_t reads_bytes;
-  const char *maf;
+  const char *maf;          /* MAF blocks, or with option "align" SAM alignment lines (no header) */
   int64_t maf_bytes;
   int64_t first_read, n_reads;   /* 1-based id of the first read, number of reads            */
   int64_t bases;                 /* emitted read bases in this chunk, all passes             */
@@ -195,6 +195,9 @@ int pbsim_cuda_set_model(pbsim_engine *e, const pbsim_model *m);
 /* replaces: get_genome_seq's genome.seq / genome.hp (pbsim.cpp:1032-1065): uploads the ASCII
  * sequence, upper-cases, computes homopolymer lengths, packs to 2 bits per base */
 int pbsim_cuda_set_sequence(pbsim_engine *e, const pbsim_sequence *s);
+/* RNAME of the alignment lines of the current WGS sequence (option "align"); required before simulate_begin then.
+ * set_sequence and set_synthetic_sequence forget it.  1 to 4096 printable characters, no whitespace. */
+int pbsim_cuda_set_sequence_name(pbsim_engine *e, const char *name);
 /* replaces: the per-sequence ingest of simulate_by_{qshmm,errhmm}_{trans,templ} (upper-casing with the
  * reference's first-base quirk, homopolymer lengths per sequence) for a whole set at once; needs set_model
  * first (which of the four functions is restated depends on the method).  After it, simulate_begin runs
@@ -247,6 +250,11 @@ int pbsim_cuda_device_timer(pbsim_engine *e, int stop, double *ms);
  * "bam" (1: with pass_num > 1 the reads stream holds BAM alignment records — the binary form of the reference's SAM
  * lines, what its `samtools view -b` child writes (pbsim.cpp:715-722) — and, with "deflate", BGZF blocks; the caller
  * adds the BAM header block in front and the BGZF end-of-file block behind; default 0),
+ * "align" (1: the second stream holds one SAM alignment line per (read, pass) instead of its MAF block: QNAME as in
+ * the reads stream, FLAG 0 / 16 (4: no match or substitution column), RNAME (WGS: pbsim_cuda_set_sequence_name; sets:
+ * the sequence's id), 1-based POS, MAPQ 60, CIGAR of =, X, I, D in reference order (insertions in front of the first
+ * and behind the last = / X column become S, deletions there are dropped), RNEXT * PNEXT 0 TLEN 0, SEQ and QUAL in
+ * reference orientation, NM:i; no header lines; not with "bam"; default 0),
  * "sample_spec" (--method sample; 1 (default): every copy of a pool entry is first simulated in its own thread at
  * the entry's length and only the copies that follow a shorter read are redone as chains; 0: one thread walks all
  * copies of an entry; results are identical either way; with "segments" the speculative pass of reads of at least

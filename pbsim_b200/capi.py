@@ -175,6 +175,7 @@ ENGINE_EXPORTS = [
     "pbsim_cuda_update_hp_del_bias", "pbsim_cuda_get_sequence_ascii", "pbsim_cuda_get_hpfreq", "pbsim_cuda_simulate_begin", "pbsim_cuda_next_chunk",
     "pbsim_cuda_next_chunk_device", "pbsim_cuda_simulate_end", "pbsim_cuda_stats_device_block",
     "pbsim_cuda_last_chunk_info", "pbsim_cuda_device_timer", "pbsim_cuda_set_option",
+    "pbsim_cuda_set_sequence_name",
 ]
 
 
@@ -207,6 +208,8 @@ def declare_engine(L):
     L.pbsim_cuda_destroy.argtypes = [C.c_void_p]
     L.pbsim_cuda_set_model.argtypes = [C.c_void_p, C.POINTER(Model)]
     L.pbsim_cuda_set_sequence.argtypes = [C.c_void_p, C.POINTER(Sequence)]
+    L.pbsim_cuda_set_sequence_name.restype = C.c_int
+    L.pbsim_cuda_set_sequence_name.argtypes = [C.c_void_p, C.c_char_p]
     L.pbsim_cuda_set_seqset.argtypes = [C.c_void_p, C.POINTER(SeqSet)]
     L.pbsim_cuda_set_pool.argtypes = [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64]
     L.pbsim_cuda_set_synthetic_sequence.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_uint64]

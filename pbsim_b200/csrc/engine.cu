@@ -37,6 +37,7 @@
 #include "gz_kernels.cuh"
 #include "k0_genome.cuh"
 #include "model_image.hpp"
+#include "align.cuh"
 #include "sample_plan.hpp"
 #include "seg_kernels.cuh"
 #include "sim_kernels.cuh"
@@ -279,6 +280,9 @@ struct pbsim_engine {
   // option "deflate": host delivery hands out gzip members (gz_kernels.cuh) instead of text
   int deflate = 0;
   int bam = 0;                      // option "bam": multi-pass records are BAM alignment records, not SAM text
+  int align = 0;                    // option "align": the second stream holds SAM alignment lines, not MAF blocks
+  std::string seq_name;             // RNAME of WGS alignment lines (pbsim_cuda_set_sequence_name; reset by set_sequence)
+  DevBuf d_rname, d_aln_rec, d_aln_maf;
   OutSet gz[2];
   DevBuf d_gz_tables, d_gz_hist, d_gz_usize, d_gz_ucrc, d_gz_uoff, d_gz_usel, d_gz_sbits;
   PinnedBuf h_gz;
@@ -533,7 +537,8 @@ struct BatchResult {
 
 // slices of b_sub_u64, each n_sub + 1 long; kSliceScanIn is the input of a scan (widened counts, pass-0 lengths)
 enum U64Slice { kSliceEvOff, kSliceCkOff, kSliceScanIn, kSliceRlen0Prefix, kSliceReadsSize, kSliceMafSize, kSliceNtiles,
-                kSliceReadsOff, kSliceMafOff, kSliceTileStart, kSliceSegOff, kSliceChunkOff, kU64Slices };
+                kSliceReadsOff, kSliceMafOff, kSliceTileStart, kSliceSegOff, kSliceChunkOff, kSliceSamSize, kSliceSamOff,
+                kU64Slices };
 
 inline unsigned long long *u64_slice(pbsim_engine *e, U64Slice k) {
   return e->b_sub_u64.as<unsigned long long>() + (size_t)k * (e->B.n_sub + 1);
@@ -890,6 +895,44 @@ int quota_cut(pbsim_engine *e, BatchCtx &c, int attempt) {
   return 0;
 }
 
+// K5 (option "align"): the MAF blocks pass 2 left in d_aln_maf -> SAM alignment lines in the output set's second stream
+int align_batch(pbsim_engine *e, const EmitArgs &EA, BatchResult *out) {
+  const uint32_t n = EA.n_sub;
+  unsigned long long *sam_size = u64_slice(e, kSliceSamSize), *sam_off = u64_slice(e, kSliceSamOff);
+  CK(cudaMemsetAsync(sam_size + n, 0, 8, e->st));
+  CK(e->d_aln_rec.ensure((size_t)n * sizeof(AlnRec) + 64));
+  AlnArgs A;
+  A.S = EA.S;
+  A.B = EA.B;
+  A.P = EA.P;
+  A.n_sub = n;
+  A.lay = EA.lay;
+  A.reads_off = EA.reads_off;
+  A.maf_off = EA.maf_off;
+  A.reads = EA.out_reads;
+  A.maf = EA.out_maf;
+  A.rname = e->d_rname.as<uint8_t>();
+  A.rname_len = (uint32_t)e->seq_name.size();
+  A.rec = e->d_aln_rec.as<AlnRec>();
+  A.sam_off = (const uint64_t *)sam_off;
+  A.sam = nullptr;
+  const uint32_t grid = nblk(n, 8);
+  k_aln_sizes<<<grid, 256, 0, e->st>>>(A, (uint64_t *)sam_size);
+  e->launches++;
+  int rc;
+  if ((rc = excl_scan(e, sam_size, sam_off, n + 1))) return rc;
+  unsigned long long *hctrl = host_ctrl(e);
+  if (peek(e, hctrl + 11, sam_off + n, 8)) return PBSIM_E_CUDA;
+  CK(cudaStreamSynchronize(e->st));
+  out->maf_bytes = hctrl[11];
+  pbsim_engine::OutSet &O = e->out[e->cur_set];
+  CK(O.maf.ensure((size_t)out->maf_bytes + 256));
+  A.sam = O.maf.as<uint8_t>();
+  k_aln_write<<<grid, 256, 0, e->st>>>(A);
+  e->launches++;
+  return 0;
+}
+
 // K4 record sizes, offsets and text of the reads before the cut, K6 their statistics, and the read-back of their
 // accuracies and lengths
 int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
@@ -936,7 +979,9 @@ int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
   const uint64_t n_tiles = hctrl[10];
   pbsim_engine::OutSet &O = e->out[e->cur_set];
   CK(O.reads.ensure((size_t)out->reads_bytes + 256));
-  CK(O.maf.ensure((size_t)out->maf_bytes + 256));
+  // option "align": the MAF blocks go to a scratch stream, from which k_aln_* write the alignment lines into O.maf
+  DevBuf &maf_buf = e->align ? e->d_aln_maf : O.maf;
+  CK(maf_buf.ensure((size_t)out->maf_bytes + 256));
 
   // ---- K4 emit
   EmitArgs EA;
@@ -959,7 +1004,7 @@ int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
   EA.keys.init(e->run.seed, (uint32_t)e->seq_num);
   EA.philox = c.replay ? 0u : 1u;
   EA.out_reads = O.reads.as<uint8_t>();
-  EA.out_maf = O.maf.as<uint8_t>();
+  EA.out_maf = maf_buf.as<uint8_t>();
   if (n_tiles > 0) {
     int dev_sms = 148;
     cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, e->device);
@@ -986,6 +1031,7 @@ int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
       }
       e->launches++;
     }
+    if (e->align && (rc = align_batch(e, EA, out))) return rc;
     CK(cudaEventRecord(e->ev_k[3], e->st));
     e->launches++;
   }
@@ -1728,7 +1774,23 @@ int pbsim_cuda_set_sequence(pbsim_engine *e, const pbsim_sequence *s) {
   const int rc = upload_ascii(e, s->bases, s->len);
   if (rc) return rc;
   e->strategy = PBSIM_STRATEGY_WGS;
+  e->seq_name.clear();
   return finish_sequence_ingest(e, s->len, s->seq_num, s->hp_del_bias);
+}
+
+int pbsim_cuda_set_sequence_name(pbsim_engine *e, const char *name) {
+  if (!e || !name) return PBSIM_E_INVALID;
+  CK(cudaSetDevice(e->device));
+  const size_t n = strlen(name);
+  if (n < 1 || n > 4096) return fail(e, PBSIM_E_INVALID, "sequence name must have 1 to 4096 characters");
+  for (size_t i = 0; i < n; ++i)
+    if ((unsigned char)name[i] <= ' ' || (unsigned char)name[i] > '~')
+      return fail(e, PBSIM_E_INVALID, "sequence name must be printable characters without whitespace");
+  if (e->running) return fail(e, PBSIM_E_INVALID, "the sequence name cannot change during a run");
+  CK(e->d_rname.ensure(n + 16));
+  CK(cudaMemcpy(e->d_rname.p, name, n, cudaMemcpyHostToDevice));
+  e->seq_name.assign(name, n);
+  return 0;
 }
 
 int pbsim_cuda_set_seqset(pbsim_engine *e, const pbsim_seqset *s) {
@@ -1820,6 +1882,7 @@ int pbsim_cuda_set_synthetic_sequence(pbsim_engine *e, int64_t len, int32_t seq_
   e->launches++;
   double bias[12] = {0, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 0};
   e->strategy = PBSIM_STRATEGY_WGS;
+  e->seq_name.clear();
   return finish_sequence_ingest(e, len, seq_num, bias);
 }
 
@@ -1854,6 +1917,9 @@ int pbsim_cuda_simulate_begin(pbsim_engine *e, const pbsim_run *run) {
   if (!e->model_set || !e->seq_set) return fail(e, PBSIM_E_INVALID, "set_model and set_sequence must precede simulate_begin");
   if (run->rng_mode == PBSIM_RNG_REPLAY && (!run->replay_draws || !run->replay_starts || run->replay_nsubreads < 1))
     return fail(e, PBSIM_E_INVALID, "replay mode needs the draw log and the subread starts");
+  if (e->align && e->bam) return fail(e, PBSIM_E_INVALID, "options align and bam cannot be combined (alignment lines are SAM text)");
+  if (e->align && e->strategy == PBSIM_STRATEGY_WGS && e->seq_name.empty())
+    return fail(e, PBSIM_E_INVALID, "option align needs pbsim_cuda_set_sequence_name after set_sequence (the RNAME of the records)");
   // a run abandoned without simulate_end: its producer thread must be gone before any run state changes
   stop_producer(e);
   CK(cudaStreamSynchronize(e->st_copy));  // a piece of that run may still be on its way into the staging buffers
@@ -2049,6 +2115,11 @@ int pbsim_cuda_set_option(pbsim_engine *e, const char *name, int64_t value) {
   if (!strcmp(name, "bam")) {
     if (e->running) return fail(e, PBSIM_E_INVALID, "bam cannot change during a run");
     e->bam = value != 0;
+    return 0;
+  }
+  if (!strcmp(name, "align")) {
+    if (e->running) return fail(e, PBSIM_E_INVALID, "align cannot change during a run");
+    e->align = value != 0;
     return 0;
   }
   if (!strcmp(name, "deflate")) {

@@ -72,6 +72,7 @@ struct Options {
   int rank = 0, world = 1;   // one process per GPU: process `rank` of `world` simulates the sequences n with
                              // (n - 1) % world == rank (their output files are independent of everything else)
   std::string gzip = "gpu";  // who writes the gzip members: the GPU (gz_kernels.cuh) or zlib threads on the host
+  std::string align = "maf"; // the second file: MAF blocks (.maf.gz) or SAM alignment lines (.aln.sam.gz)
 };
 
 std::thread *g_background = nullptr;  // a thread that must have ended before the process exits (CUDA start-up)
@@ -768,7 +769,10 @@ void print_help() {
           "  --rank R --world N   one process per GPU: this process simulates the sequences n with (n-1) %% N == R\n"
           "                       (WGS; every process reads the whole genome, files are written per sequence).\n"
           "  --gzip               gpu (default): gzip members / BGZF blocks are written on the GPU (multi-pass\n"
-          "                       output is <prefix>_NNNN.bam) | host: zlib threads (multi-pass: .sam.gz).\n\n"
+          "                       output is <prefix>_NNNN.bam) | host: zlib threads (multi-pass: .sam.gz).\n"
+          "  --align              maf (default): alignments as MAF, <prefix>_NNNN.maf.gz | sam: each read's true\n"
+          "                       alignment as a SAM line with a CIGAR, <prefix>_NNNN.aln.sam.gz (with --pass-num > 1\n"
+          "                       it needs --gzip host).\n\n"
           " [options for transcriptome / template sequencing]\n\n"
           "  --strategy           trans | templ\n"
           "  --transcript         transcript table: id, plus count, minus count, sequence (tab separated).\n"
@@ -812,7 +816,8 @@ int main(int argc, char **argv) {
       // engine-only
       {"gpu", 1, nullptr, 0},        {"rng", 1, nullptr, 0},            {"replay-draws", 1, nullptr, 0},
       {"replay-marks", 1, nullptr, 0}, {"threads", 1, nullptr, 0},      {"gzip", 1, nullptr, 0},
-      {"rank", 1, nullptr, 0},       {"world", 1, nullptr, 0},          {nullptr, 0, nullptr, 0}};
+      {"rank", 1, nullptr, 0},       {"world", 1, nullptr, 0},          {"align", 1, nullptr, 0},
+      {nullptr, 0, nullptr, 0}};
   int opt, idx = 0;
   while ((opt = getopt_long(argc, argv, "", long_options, &idx)) != -1) {
     if (opt != 0) exit(-1);
@@ -908,6 +913,10 @@ int main(int argc, char **argv) {
       case 28:
         if (!strcmp(a, "gpu") || !strcmp(a, "host")) o.gzip = a;
         else die("ERROR (gzip: %s): Acceptable value: gpu, host.\n", a);
+        break;
+      case 31:
+        if (!strcmp(a, "maf") || !strcmp(a, "sam")) o.align = a;
+        else die("ERROR (align: %s): Acceptable value: maf, sam.\n", a);
         break;
       default: break;
     }
@@ -1172,9 +1181,17 @@ int main(int argc, char **argv) {
   // <stem>.sam.gz with --gzip host
   const bool bam = o.pass_num > 1 && o.gzip == "gpu";
   if (pbsim_cuda_set_option(eng, "bam", bam ? 1 : 0) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
-  auto simulate_to_files = [&](const std::string &stem, const std::string &pu, int64_t len_quota) {
+  const bool align = o.align == "sam";
+  if (align && bam) die("ERROR: --align sam with --pass-num > 1 needs --gzip host (BAM reads and SAM alignment lines are not written together).\n");
+  if (pbsim_cuda_set_option(eng, "align", align ? 1 : 0) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
+  // sq: the @SQ lines of the alignment file (--align sam)
+  auto simulate_to_files = [&](const std::string &stem, const std::string &pu, int64_t len_quota, const std::string &sq) {
     GzipWriter reads_out((stem + (o.pass_num == 1 ? ".fq.gz" : (bam ? ".bam" : ".sam.gz"))).c_str(), std::max(1, threads / 2));
-    GzipWriter maf_out((stem + ".maf.gz").c_str(), std::max(1, threads / 2));
+    GzipWriter maf_out((stem + (align ? ".aln.sam.gz" : ".maf.gz")).c_str(), std::max(1, threads / 2));
+    if (align) {
+      const std::string h = "@HD\tVN:1.6\tSO:unknown\n" + sq + "@PG\tID:pbsim\tPN:pbsim\n";
+      maf_out.submit(h.data(), h.size());
+    }
     if (o.pass_num > 1) {  // SAM header (:721-722, :781-782)
       char hdr[1024];
       int m = snprintf(hdr, sizeof hdr,
@@ -1298,7 +1315,10 @@ int main(int argc, char **argv) {
       pbsim_host_hp_del_bias(o.hp_del_bias, f, ss.hp_del_bias);
       if (pbsim_cuda_set_seqset(eng, &ss) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
     }
-    const pbsim_stats st = simulate_to_files(o.prefix, o.id_prefix, 0);
+    std::string sq;
+    for (size_t t = 0; align && t < S.ids.size(); ++t)
+      sq += "@SQ\tSN:" + S.ids[t] + "\tLN:" + std::to_string(S.start[t + 1] - S.start[t]) + "\n";
+    const pbsim_stats st = simulate_to_files(o.prefix, o.id_prefix, 0, sq);
     fprintf(stderr, ":::: Simulation stats ::::\n\n");
     fprintf(stderr, "read num. : %ld\n", (long)st.res_num);
     print_stats_tail(st);
@@ -1308,6 +1328,11 @@ int main(int argc, char **argv) {
 
   // ---- hp-del-bias (main :673-697)
   int64_t hp11_running = 0;
+  auto seq_name = [&](size_t num) {  // RNAME / @SQ SN of sequence num: the first word of its FASTA header
+    const std::string &id = seqs[num - 1].id;
+    const size_t e = id.find_first_of(" \t\r\v\f");
+    return id.substr(0, e);
+  };
   auto ingest = [&](size_t num, const double b[12], int64_t hpfreq[12]) {
     // the split pass kept the text (identical to what genome_seq re-reads from <prefix>_NNNN.ref: the split writes
     // the body lines verbatim, :953-957)
@@ -1318,6 +1343,7 @@ int main(int argc, char **argv) {
     s.seq_num = (int32_t)num;
     memcpy(s.hp_del_bias, b, sizeof s.hp_del_bias);
     if (pbsim_cuda_set_sequence(eng, &s) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
+    if (align && pbsim_cuda_set_sequence_name(eng, seq_name(num).c_str()) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
     pbsim_cuda_get_hpfreq(eng, hpfreq);
     return (int64_t)seq.size();
   };
@@ -1343,7 +1369,8 @@ int main(int argc, char **argv) {
     char stem[4096], pu[512];
     snprintf(stem, sizeof stem, "%s_%04zu", o.prefix.c_str(), n);
     snprintf(pu, sizeof pu, "%s%zu", o.id_prefix.c_str(), n);
-    const pbsim_stats st = simulate_to_files(stem, pu, (int64_t)(o.depth * glen));  // sim.len_quota (:705)
+    const std::string sq = align ? "@SQ\tSN:" + seq_name(n) + "\tLN:" + std::to_string(glen) + "\n" : "";
+    const pbsim_stats st = simulate_to_files(stem, pu, (int64_t)(o.depth * glen), sq);  // sim.len_quota (:705)
     // print_simulation_stats (:5541-5564)
     fprintf(stderr, ":::: Simulation stats (ref.%zu) ::::\n\n", n);
     fprintf(stderr, "read num. : %ld\n", (long)st.res_num);

@@ -67,6 +67,11 @@ class Engine:
         id_start[1:] = np.cumsum([len(x) for x in names])
         return dict(n=len(seqset), bases=bases, start=start, plus=plus, minus=minus, ids=ids, id_start=id_start)
 
+    def set_sequence_name(self, name):
+        """RNAME of the alignment lines (option "align") of the current WGS sequence; set after set_sequence"""
+        self._chk(self.L.pbsim_cuda_set_sequence_name(self.h, name.encode() if isinstance(name, str) else name),
+                  "set_sequence_name")
+
     def set_seqset(self, strategy, seqset, bias):
         """strategy 'trans' | 'templ'; seqset = [(name, plus, minus, bases)] as parsed from the transcript table /
         template FASTA (pbsim.cpp:1075, :1366), or the result of pack_seqset"""
@@ -243,9 +248,12 @@ class WgsRun:
         self.hp11_running = tot[11]
         self.base_bias = capi.hp_del_bias(self.e.L, self.opt, tot)
 
-    def simulate_sequence(self, bases, seq_num, **kw):
+    def simulate_sequence(self, bases, seq_num, name=None, **kw):
+        """name: RNAME of the alignment lines (option "align")"""
         bias = list(self.base_bias)
         self.e.set_sequence(bases, seq_num, bias)
+        if name is not None:
+            self.e.set_sequence_name(name)
         f = self.e.hpfreq()
         self.hp11_running += f[11]
         bias[0] = float(np.array([self.hp11_running], dtype=np.int64).view(np.float64)[0])
