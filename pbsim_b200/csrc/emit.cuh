@@ -134,6 +134,11 @@ __device__ __forceinline__ uint32_t bam_nibble(uint8_t c) {
     case 'K': return 12u; case 'D': return 13u; case 'B': return 14u; default: return 15u;
   }
 }
+// BAM base bytes that two writers share (two bases per byte): OR the bits into the zeroed record
+__device__ __forceinline__ void atomic_or_byte(uint8_t *b, uint32_t bits) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(b);
+  atomicOr(reinterpret_cast<unsigned int *>(a & ~(uintptr_t)3), bits << (8u * (uint32_t)(a & 3u)));
+}
 // one read base into its row(s): text formats store characters; BAM packs two bases per byte (high nibble first)
 // with an atomic OR into the zeroed record, and stores the quality value itself
 template <bool BAM>
@@ -143,9 +148,7 @@ __device__ __forceinline__ void put_read_base(uint8_t *seq, uint8_t *qual, uint3
     seq[Pp] = ch;
     qual[Pp] = has_qv ? (uint8_t)(qv + 33u) : (uint8_t)'!';
   } else {
-    uint8_t *b = seq + (Pp >> 1);
-    const uintptr_t a = reinterpret_cast<uintptr_t>(b);
-    atomicOr(reinterpret_cast<unsigned int *>(a & ~(uintptr_t)3), (nib << ((Pp & 1u) ? 0u : 4u)) << (8u * (uint32_t)(a & 3u)));
+    atomic_or_byte(seq + (Pp >> 1), nib << ((Pp & 1u) ? 0u : 4u));
     qual[Pp] = has_qv ? (uint8_t)qv : (uint8_t)0;
   }
 }
@@ -385,35 +388,26 @@ __device__ __forceinline__ uint8_t comp_char(uint8_t c) {  // revcomp's compleme
   }
 }
 
+// reference bases of the generic tile path, from the ASCII copy of the genome
 struct RefFetch {
-  const uint32_t *__restrict__ pk;
   const uint8_t *__restrict__ ascii;
   uint32_t offset, wlen, minus;
-  bool slow;
   // window index r -> forward genome char, window-strand char, window-strand code, ACGT flag
   __device__ __forceinline__ void get(uint32_t r, uint8_t &gch, uint8_t &wch, uint32_t &wc, bool &acgt) const {
     const uint32_t g = minus ? offset + wlen - 1u - r : offset + r;
     const uint32_t lut = 0x54474341u;  // "ACGT"
-    if (!slow) {
-      const uint32_t gc = (__ldg(&pk[g >> 4]) >> ((g & 15u) * 2u)) & 3u;
-      wc = gc ^ (minus ? 3u : 0u);
-      gch = (uint8_t)(lut >> (8u * gc));
-      wch = (uint8_t)(lut >> (8u * wc));
-      acgt = true;
-    } else {
-      gch = __ldg(&ascii[g]);
-      uint32_t gc = 0;
-      acgt = true;
-      switch (gch) {
-        case 'A': gc = 0; break;
-        case 'C': gc = 1; break;
-        case 'G': gc = 2; break;
-        case 'T': gc = 3; break;
-        default: acgt = false; break;
-      }
-      wc = gc ^ (minus ? 3u : 0u);
-      wch = acgt ? (uint8_t)(lut >> (8u * wc)) : gch;
+    gch = __ldg(&ascii[g]);
+    uint32_t gc = 0;
+    acgt = true;
+    switch (gch) {
+      case 'A': gc = 0; break;
+      case 'C': gc = 1; break;
+      case 'G': gc = 2; break;
+      case 'T': gc = 3; break;
+      default: acgt = false; break;
     }
+    wc = gc ^ (minus ? 3u : 0u);
+    wch = acgt ? (uint8_t)(lut >> (8u * wc)) : gch;
   }
 };
 
@@ -432,7 +426,7 @@ __device__ __forceinline__ uint8_t read_base(uint32_t kind, uint32_t info, uint8
   return info >= 4u ? wch : (uint8_t)(nt4 >> (8u * info));
 }
 
-// ---- fast tile path -------------------------------------------------------------------------
+// ---- read-base codes of the staged tile path's lookup tables ------------------------------------
 // Everything in 2-bit code space (A=0 C=1 G=2 T=3, complement = ^3), converted to characters with
 // one byte-permute per output.  Substitution alphabets of set_mut (:5481-5486) as 2-bit codes:
 //   A -> T,G,C   C -> A,T,G   G -> A,T,C   T -> A,G,C      index = window code * 3 + choice
@@ -456,148 +450,13 @@ __device__ __forceinline__ uint32_t read_code(uint32_t kind, uint32_t info, uint
 constexpr uint32_t kEmitPerLane = 4;                    // entries per lane per iteration
 constexpr uint32_t kEmitStep = 32u * kEmitPerLane;      // entries per warp iteration
 
-// One tile whose reference range holds only ACGT: 4 entries per lane, one packed warp scan per 128 entries.
-template <int METHOD, bool BAM>
-__device__ __forceinline__ void emit_tile_fast(const uint8_t *__restrict__ evbase, uint32_t e0, uint32_t e1,
-                                               const uint32_t *__restrict__ pk, uint32_t offset, uint32_t wlen,
-                                               uint32_t minus, uint32_t ncol, uint32_t C0, uint32_t R0, uint32_t P0,
-                                               uint8_t *__restrict__ seq, uint8_t *__restrict__ qual,
-                                               uint8_t *__restrict__ mref, uint8_t *__restrict__ mread, uint32_t lane,
-                                               const uint8_t *lut_s /* read_code by kind<<5 | info<<2 | window code */) {
-  const uint32_t flip = minus ? 3u : 0u;
-  // ---- 4 entries per lane and iteration (tile starts are 16-byte aligned, so the vector load is aligned; entries
-  //      past e1 are masked: the slot behind them is padded scratch).  The entries of the NEXT iteration are
-  //      requested before the current ones are processed, so the DRAM latency overlaps the formatting work.
-  auto load_entries = [&](uint32_t i) -> uint2 {
-    const uint32_t eb = i + lane * kEmitPerLane;
-    if (METHOD == PBSIM_METHOD_QSHMM) return __ldg(reinterpret_cast<const uint2 *>(evbase + 2ull * eb));
-    return make_uint2(__ldg(reinterpret_cast<const uint32_t *>(evbase + eb)), 0u);
-  };
-  uint2 nxt = load_entries(e0);
-  for (uint32_t i = e0; i < e1; i += kEmitStep) {
-    const uint32_t eb = i + lane * kEmitPerLane;
-    const uint2 v = nxt;
-    if (i + kEmitStep < e1) nxt = load_entries(i + kEmitStep);
-    uint32_t raw[kEmitPerLane];
-    if (METHOD == PBSIM_METHOD_QSHMM) {
-      raw[0] = v.x & 0xFFFFu; raw[1] = v.x >> 16; raw[2] = v.y & 0xFFFFu; raw[3] = v.y >> 16;
-    } else {
-      raw[0] = v.x & 0xFFu; raw[1] = (v.x >> 8) & 0xFFu; raw[2] = (v.x >> 16) & 0xFFu; raw[3] = v.x >> 24;
-    }
-    uint32_t kind[kEmitPerLane], info[kEmitPerLane], nd[kEmitPerLane], isb[kEmitPerLane], adv[kEmitPerLane];
-    uint32_t lb = 0, la = 0, ld = 0;  // this lane's totals: read bases, ref advances by bases, deletions
-#pragma unroll
-    for (uint32_t k = 0; k < kEmitPerLane; ++k) {
-      const bool valid = eb + k < e1;
-      const uint32_t v = raw[k];
-      if (METHOD == PBSIM_METHOD_QSHMM) {
-        kind[k] = (v >> 7) & 3u;
-        info[k] = (v >> 9) & 7u;
-        const bool cont = kind[k] == 3u;
-        nd[k] = valid ? (cont ? ((v & 0x7Fu) | ((v >> 9) << 7)) : (v >> 12)) : 0u;
-        isb[k] = (valid && !cont) ? 1u : 0u;
-        adv[k] = (isb[k] && kind[k] != PB_KIND_INS) ? 1u : 0u;
-      } else {
-        kind[k] = v & 3u;
-        info[k] = (v >> 2) & 7u;
-        nd[k] = (valid && kind[k] == PB_KIND_DEL) ? 1u : 0u;
-        isb[k] = (valid && kind[k] != PB_KIND_DEL) ? 1u : 0u;
-        adv[k] = (isb[k] && kind[k] != PB_KIND_INS) ? 1u : 0u;
-      }
-      lb += isb[k];
-      la += adv[k];
-      ld += nd[k];
-    }
-    // ---- one warp scan over the packed per-lane totals: bases (8 bit) | advances (8 bit) | deletions (16 bit)
-    // deletion counts that do not fit (long continuation runs) take the wide scan
-    uint32_t pre_b, pre_a, pre_d, tot_b, tot_a, tot_d;
-    if (__any_sync(0xFFFFFFFFu, ld >= 2048u)) {
-      uint32_t xb = lb, xa = la, xd = ld;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t yb = __shfl_up_sync(0xFFFFFFFFu, xb, o), ya = __shfl_up_sync(0xFFFFFFFFu, xa, o),
-                       yd = __shfl_up_sync(0xFFFFFFFFu, xd, o);
-        if (lane >= (uint32_t)o) { xb += yb; xa += ya; xd += yd; }
-      }
-      tot_b = __shfl_sync(0xFFFFFFFFu, xb, 31); tot_a = __shfl_sync(0xFFFFFFFFu, xa, 31);
-      tot_d = __shfl_sync(0xFFFFFFFFu, xd, 31);
-      pre_b = xb - lb; pre_a = xa - la; pre_d = xd - ld;
-    } else {
-      const uint32_t mine = lb | (la << 8) | (ld << 16);
-      uint32_t x = mine;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, x, o);
-        if (lane >= (uint32_t)o) x += y;
-      }
-      const uint32_t tot = __shfl_sync(0xFFFFFFFFu, x, 31);
-      const uint32_t pre = x - mine;
-      pre_b = pre & 0xFFu; pre_a = (pre >> 8) & 0xFFu; pre_d = pre >> 16;
-      tot_b = tot & 0xFFu; tot_a = (tot >> 8) & 0xFFu; tot_d = tot >> 16;
-    }
-    uint32_t Pp = P0 + pre_b, Rr = R0 + pre_a + pre_d, Cc = C0 + pre_b + pre_d;
-    // ---- reference bases this lane may need: window positions Rr .. Rr+3 (+ deletions, fetched on demand)
-#pragma unroll
-    for (uint32_t k = 0; k < kEmitPerLane; ++k) {
-      if (METHOD == PBSIM_METHOD_ERRHMM) {
-        // errhmm: an entry is one alignment column, a deletion included, so a deleted column takes the same
-        // straight-line path as a base (no per-entry deletion loop, which runs at 2 of 32 lanes)
-        if (isb[k] | nd[k]) {
-          const uint32_t g = minus ? offset + wlen - 1u - Rr : offset + Rr;
-          const uint32_t gc = (__ldg(&pk[g >> 4]) >> ((g & 15u) * 2u)) & 3u;
-          const uint32_t col = minus ? ncol - 1u - Cc : Cc;
-          if (isb[k]) {
-            const uint32_t rc = lut_s[(kind[k] << 5) | (info[k] << 2) | (gc ^ flip)];
-            put_read_base<BAM>(seq, qual, Pp, code_char(rc), 1u << rc, 0u, false);
-            mread[col] = code_char(rc ^ flip);
-            mref[col] = (kind[k] == PB_KIND_INS) ? (uint8_t)'-' : code_char(gc);
-            ++Pp;
-          } else {
-            mread[col] = '-';
-            mref[col] = code_char(gc);
-          }
-          ++Cc;
-          Rr += adv[k] + nd[k];
-        }
-        continue;
-      }
-      if (isb[k]) {
-        const uint32_t g = minus ? offset + wlen - 1u - Rr : offset + Rr;
-        const uint32_t gc = (__ldg(&pk[g >> 4]) >> ((g & 15u) * 2u)) & 3u;
-        const uint32_t wc = gc ^ flip;
-        const uint32_t rc = lut_s[(kind[k] << 5) | (info[k] << 2) | wc];
-        put_read_base<BAM>(seq, qual, Pp, code_char(rc), 1u << rc, raw[k] & 0x7Fu, METHOD == PBSIM_METHOD_QSHMM);
-        const uint32_t col = minus ? ncol - 1u - Cc : Cc;
-        mread[col] = code_char(rc ^ flip);
-        mref[col] = (kind[k] == PB_KIND_INS) ? (uint8_t)'-' : code_char(gc);
-        ++Pp;
-        ++Cc;
-        Rr += adv[k];
-      }
-      if (nd[k] != 0u) {
-        for (uint32_t j = 0; j < nd[k]; ++j) {
-          const uint32_t g = minus ? offset + wlen - 1u - Rr : offset + Rr;
-          const uint32_t gc = (__ldg(&pk[g >> 4]) >> ((g & 15u) * 2u)) & 3u;
-          const uint32_t col = minus ? ncol - 1u - Cc : Cc;
-          mread[col] = '-';
-          mref[col] = code_char(gc);
-          ++Cc;
-          ++Rr;
-        }
-      }
-    }
-    P0 += tot_b;
-    R0 += tot_a + tot_d;
-    C0 += tot_b + tot_d;
-  }
-}
-
 // Everything the row kernel needs to know about a tile, gathered once by k_tile_desc (one THREAD per tile: the
 // dependent loads through tile -> sub-read -> plan / layout / checkpoints run with full memory-level parallelism
 // there instead of as a serial prologue in front of every tile).
 struct TileDesc {
   uint64_t ev_off;          // byte offset of the tile's first entry in the event arena
-  uint64_t o_seq, o_qual;   // byte offsets in the reads stream of the tile's first read base / quality
+  uint64_t o_seq, o_qual;   // byte offsets in the reads stream of the tile's first read base / quality (BAM: o_seq
+                            // is the nibble offset of the base, two per byte, high nibble first)
   uint64_t o_ref, o_read;   // byte offsets in the MAF stream of the tile's first column (file order) in both rows
   uint32_t e1;              // entries of the tile
   uint32_t Pn, Cn, Rn;      // read bases, MAF columns and window bases it covers
@@ -665,18 +524,54 @@ __device__ __forceinline__ void flush_row(const uint8_t *buf, uint8_t *__restric
   if (tail_start + lane < total) g0[tail_start + lane] = buf[tail_start + lane];
 }
 
+// 8 BAM base codes, one per byte of x and y -> 4 bytes of two bases each (high nibble first); codes outside the
+// tile are whatever the staging row held, hence the masks
+__device__ __forceinline__ uint32_t pack_codes(uint32_t x, uint32_t y) {
+  x &= 0x0F0F0F0Fu;
+  y &= 0x0F0F0F0Fu;
+  return __byte_perm((x << 4) | (x >> 8), (y << 4) | (y >> 8), 0x6420u);
+}
+
+// BAM read bases: buf[shift + i] holds the code of base i, g0 the 16-byte aligned byte whose high nibble is buf[0].
+// The codes are packed two per byte in place; the bytes that hold two bases of the tile go out through flush_row, a
+// first / last byte that the tile shares with its neighbour (odd start / end) gets its nibble with an atomic OR
+// into the zeroed record.
+__device__ __forceinline__ void flush_nibbles(uint8_t *buf, uint8_t *__restrict__ g0, uint32_t n, uint32_t shift,
+                                              uint32_t lane) {
+  if (n == 0u) return;
+  const uint32_t total = shift + n;
+  for (uint32_t j0 = 0; j0 < total; j0 += 1024u) {  // 32 codes per lane -> 16 bytes, written over codes already read
+    const uint32_t j = j0 + lane * 32u;
+    uint4 a = make_uint4(0u, 0u, 0u, 0u), b = a;
+    if (j < total) {
+      a = *reinterpret_cast<const uint4 *>(buf + j);
+      b = *reinterpret_cast<const uint4 *>(buf + j + 16u);
+    }
+    __syncwarp();
+    if (j < total)
+      *reinterpret_cast<uint4 *>(buf + j / 2u) =
+          make_uint4(pack_codes(a.x, a.y), pack_codes(a.z, a.w), pack_codes(b.x, b.y), pack_codes(b.z, b.w));
+  }
+  __syncwarp();
+  const uint32_t lo = (shift + 1u) >> 1, hi = total >> 1;  // bytes [lo, hi) hold two bases of the tile
+  flush_row(buf + (lo & ~15u), g0 + lo, hi - lo, lo & 15u, lane);
+  if (lane == 0u && (shift & 1u)) atomic_or_byte(g0 + (shift >> 1), buf[shift >> 1] & 0x0Fu);
+  if (lane == 1u && (total & 1u)) atomic_or_byte(g0 + (total >> 1), buf[total >> 1] & 0xF0u);
+}
+
 // byte LUTs of the staged path, index = (kind | info << 2) << 2 | window code of the current reference base
-// (kind 3 = errhmm deletion column).  seq: the read base; mread / mref: the MAF characters for the plus ([0]) and
-// the minus strand ([1], complemented because the rows are mirrored back).
+// (kind 3 = errhmm deletion column).  seq: the read base (BAM: its 4-bit code 1 << code); mread / mref: the MAF
+// characters for the plus ([0]) and the minus strand ([1], complemented because the rows are mirrored back).
 struct EmitLuts {
   uint8_t seq[128];
   uint8_t mread[2][128];
   uint8_t mref[2][128];
 };
+template <bool BAM>
 __device__ __forceinline__ void build_emit_luts(EmitLuts &L, uint32_t t) {  // t = 0 .. 127
   const uint32_t wc = t & 3u, kind = (t >> 2) & 3u, info = (t >> 4) & 7u;
   const uint32_t rc = read_code(kind == 3u ? 0u : kind, info, wc);
-  L.seq[t] = code_char(rc);
+  L.seq[t] = BAM ? (uint8_t)(1u << rc) : code_char(rc);
   for (uint32_t f = 0; f < 2u; ++f) {
     const uint32_t flip = f ? 3u : 0u;
     L.mread[f][t] = kind == 3u ? (uint8_t)'-' : code_char(rc ^ flip);
@@ -684,16 +579,19 @@ __device__ __forceinline__ void build_emit_luts(EmitLuts &L, uint32_t t) {  // t
   }
 }
 
-// One tile whose reference range holds only ACGT, text records (Cn <= kStageCols, Pn <= PB_TILE).
-template <int METHOD>
+// One tile whose reference range holds only ACGT (Cn <= kStageCols, Pn <= PB_TILE).  BAM: g_seq is the byte of the
+// tile's first base, seq_odd 1 when that base is its low nibble; qualities are the values themselves.
+template <int METHOD, bool BAM>
 __device__ __forceinline__ void emit_tile_staged(EmitStage &S, const EmitLuts &LU, const uint8_t *__restrict__ evbase,
                                                  uint32_t e1, const uint32_t *__restrict__ pk, uint32_t glen_words,
                                                  uint32_t wpos, uint32_t minus, uint32_t Pn, uint32_t Cn, uint32_t Rn,
-                                                 uint8_t *__restrict__ g_seq, uint8_t *__restrict__ g_qual,
+                                                 uint8_t *__restrict__ g_seq, uint32_t seq_odd, uint8_t *__restrict__ g_qual,
                                                  uint8_t *__restrict__ g_ref, uint8_t *__restrict__ g_read, uint32_t lane) {
   const uint32_t e0 = 0;
-  // the offsets (modulo 16) the staging rows of the four fragments start at
-  const uint32_t sh_s = (uint32_t)(reinterpret_cast<uintptr_t>(g_seq) & 15u);
+  constexpr uint32_t qoff = BAM ? 0u : 33u;  // '!' + quality value
+  // the offsets (modulo 16) the staging rows of the four fragments start at; BAM bases: the nibble offset modulo 32
+  const uint32_t sh_s = BAM ? 2u * (uint32_t)(reinterpret_cast<uintptr_t>(g_seq) & 15u) + seq_odd
+                            : (uint32_t)(reinterpret_cast<uintptr_t>(g_seq) & 15u);
   const uint32_t sh_q = (uint32_t)(reinterpret_cast<uintptr_t>(g_qual) & 15u);
   const uint32_t sh_r = (uint32_t)(reinterpret_cast<uintptr_t>(g_ref) & 15u);
   const uint32_t sh_m = (uint32_t)(reinterpret_cast<uintptr_t>(g_read) & 15u);
@@ -785,7 +683,7 @@ __device__ __forceinline__ void emit_tile_staged(EmitStage &S, const EmitLuts &L
         for (uint32_t k = 0; k < kEmitPerLane; ++k) {
           const uint32_t t = idx[k] | (bits & 3u);
           S.seq[sh_s + op + k] = LU.seq[t];
-          S.qual[sh_q + op + k] = (uint8_t)((raw[k] & 0x7Fu) + 33u);
+          S.qual[sh_q + op + k] = (uint8_t)((raw[k] & 0x7Fu) + qoff);
           S.mread[oc + d_read] = LU.mread[0][t + moff];
           S.mref[oc] = LU.mref[0][t + moff];
           oc += (uint32_t)cdir;
@@ -818,7 +716,7 @@ __device__ __forceinline__ void emit_tile_staged(EmitStage &S, const EmitLuts &L
           const bool isb = nd[k] == 0u;
           if (isb) {
             S.seq[sh_s + op] = LU.seq[t];
-            S.qual[sh_q + op] = '!';
+            S.qual[sh_q + op] = (uint8_t)qoff;
           }
           S.mread[oc + d_read] = LU.mread[0][t + moff];
           S.mref[oc] = LU.mref[0][t + moff];
@@ -876,7 +774,7 @@ __device__ __forceinline__ void emit_tile_staged(EmitStage &S, const EmitLuts &L
       if (isb[k]) {
         const uint32_t t = ((kind[k] | (info[k] << 2)) << 2) | (codes_at(Rr) & 3u);
         S.seq[sh_s + Pp] = LU.seq[t];
-        S.qual[sh_q + Pp] = METHOD == PBSIM_METHOD_QSHMM ? (uint8_t)((raw[k] & 0x7Fu) + 33u) : (uint8_t)'!';
+        S.qual[sh_q + Pp] = METHOD == PBSIM_METHOD_QSHMM ? (uint8_t)((raw[k] & 0x7Fu) + qoff) : (uint8_t)qoff;
         S.mread[o_ref + Cc * (uint32_t)cdir + d_read] = LU.mread[0][t + moff];
         S.mref[o_ref + Cc * (uint32_t)cdir] = LU.mref[0][t + moff];
         ++Pp;
@@ -895,7 +793,8 @@ __device__ __forceinline__ void emit_tile_staged(EmitStage &S, const EmitLuts &L
     Ct += (tot & 0xFFu) + (tot >> 16);
   }
   __syncwarp();
-  flush_row(S.seq, g_seq, Pn, sh_s, lane);
+  if (BAM) flush_nibbles(S.seq, g_seq - (sh_s >> 1), Pn, sh_s, lane);
+  else flush_row(S.seq, g_seq, Pn, sh_s, lane);
   flush_row(S.qual, g_qual, Pn, sh_q, lane);
   flush_row(S.mref, g_ref, Cn, sh_r, lane);
   flush_row(S.mread, g_read, Cn, sh_m, lane);
@@ -1047,7 +946,7 @@ __global__ void k_tile_desc(const __grid_constant__ EmitArgs A, uint32_t *tile_s
     const uint64_t rd = A.reads_off[s], mf = A.maf_off[s];
     d.ev_off = (A.B.ev_off[s] + (g.segmented ? (uint64_t)tile * PB_SEG_STRIDE : (uint64_t)g.e0)) *
                (METHOD == PBSIM_METHOD_QSHMM ? 2ull : 1ull);
-    d.o_seq = rd + L.seq_rel + g.c0.read;
+    d.o_seq = A.P.sam == 2u ? 2ull * (rd + L.seq_rel) + g.c0.read : rd + L.seq_rel + g.c0.read;
     d.o_qual = rd + L.qual_rel + g.c0.read;
     const uint32_t cfirst = minus ? ncol - g.c0.col - g.Cn : g.c0.col;   // first MAF column (file order) of the tile
     d.o_ref = mf + L.refrow_rel + cfirst;
@@ -1065,10 +964,10 @@ __global__ void k_tile_desc(const __grid_constant__ EmitArgs A, uint32_t *tile_s
   dst[0] = src[0]; dst[1] = src[1]; dst[2] = src[2]; dst[3] = src[3];
 }
 
-// The ROW kernel of pass 2 (text records): one warp per tile, everything it needs in the tile's descriptor.
+// The ROW kernel of pass 2 (text and BAM records): one warp per tile, everything it needs in the tile's descriptor.
 // Tiles that touch exceptional bases or are too wide for the staging rows are left to k_emit, as are the record
-// headers, the SAM ip / pw arrays and BAM records.  Kept small on purpose: the loop must live in the instruction cache.
-template <int METHOD>
+// headers and the SAM ip / pw arrays.  Kept small on purpose: the loop must live in the instruction cache.
+template <int METHOD, bool BAM>
 __global__ void __launch_bounds__(kEmitThreads, 4) k_emit_rows(const TileDesc *__restrict__ desc, uint64_t n_tiles,
                                                               const uint8_t *__restrict__ ev,
                                                               const uint32_t *__restrict__ pk, uint32_t glen_words,
@@ -1076,7 +975,7 @@ __global__ void __launch_bounds__(kEmitThreads, 4) k_emit_rows(const TileDesc *_
                                                               uint8_t *__restrict__ out_maf) {
   __shared__ __align__(16) EmitStage stage[kEmitWarps];
   __shared__ EmitLuts luts;
-  if (threadIdx.x < 128u) build_emit_luts(luts, threadIdx.x);
+  if (threadIdx.x < 128u) build_emit_luts<BAM>(luts, threadIdx.x);
   __syncthreads();
   const uint32_t lane = threadIdx.x & 31u;
   const uint64_t warp0 = (uint64_t)blockIdx.x * kEmitWarps + (threadIdx.x >> 5);
@@ -1089,28 +988,25 @@ __global__ void __launch_bounds__(kEmitThreads, 4) k_emit_rows(const TileDesc *_
     const uint64_t ev_off = (uint64_t)d0.x | ((uint64_t)d0.y << 32), o_seq = (uint64_t)d0.z | ((uint64_t)d0.w << 32);
     const uint64_t o_qual = (uint64_t)d1.x | ((uint64_t)d1.y << 32), o_ref = (uint64_t)d1.z | ((uint64_t)d1.w << 32);
     const uint64_t o_read = (uint64_t)d2.x | ((uint64_t)d2.y << 32);
-    emit_tile_staged<METHOD>(stage[threadIdx.x >> 5], luts, ev + ev_off, d2.z /* e1 */, pk, glen_words, d3.z /* wpos */,
-                             flags & kTileMinus, d2.w /* Pn */, d3.x /* Cn */, d3.y /* Rn */, out_reads + o_seq,
-                             out_reads + o_qual, out_maf + o_ref, out_maf + o_read, lane);
+    emit_tile_staged<METHOD, BAM>(stage[threadIdx.x >> 5], luts, ev + ev_off, d2.z /* e1 */, pk, glen_words,
+                                  d3.z /* wpos */, flags & kTileMinus, d2.w /* Pn */, d3.x /* Cn */, d3.y /* Rn */,
+                                  out_reads + (BAM ? o_seq >> 1 : o_seq), BAM ? (uint32_t)o_seq & 1u : 0u,
+                                  out_reads + o_qual, out_maf + o_ref, out_maf + o_read, lane);
   }
 }
 
-// Everything of pass 2 that is not a plain text tile: the record headers (once per sub-read), tiles that touch
-// exceptional bases or are too wide for the staging rows, the SAM ip / pw arrays, and BAM records altogether.
+// Everything of pass 2 that is not a staged tile: the record headers (once per sub-read), tiles that touch
+// exceptional bases or are too wide for the staging rows, and the SAM / BAM ip / pw arrays.
 template <int METHOD, bool BAM>
 __global__ void __launch_bounds__(kEmitThreads) k_emit(const __grid_constant__ EmitArgs A) {
-  __shared__ uint8_t lut_s[128];
-  if (threadIdx.x < 128u)
-    lut_s[threadIdx.x] = (uint8_t)read_code((threadIdx.x >> 5) & 3u, (threadIdx.x >> 2) & 7u, threadIdx.x & 3u);
-  __syncthreads();
   const uint32_t lane = threadIdx.x & 31u;
   const uint64_t warp0 = (uint64_t)blockIdx.x * kEmitWarps + (threadIdx.x >> 5);
   const uint64_t nwarps = (uint64_t)gridDim.x * kEmitWarps;
   for (uint64_t t = warp0; t < A.n_tiles; t += nwarps) {
     const uint32_t s = __ldg(&A.tile_sub[t]);
     const uint32_t tile = (uint32_t)(t - __ldg(&A.tile_start[s]));
-    // text tiles the row kernel handles: nothing to do here unless the tile opens a record or SAM arrays follow
-    const uint32_t dflags = BAM ? (kTileGeneric) : __ldg(&A.desc[t].flags);
+    // tiles the row kernel handles: nothing to do here unless the tile opens a record or SAM / BAM arrays follow
+    const uint32_t dflags = __ldg(&A.desc[t].flags);
     const bool rows_here = (dflags & (kTileGeneric | kTileWide)) != 0u;
     if (!rows_here && tile != 0u && !A.P.sam) continue;
     const uint32_t r = s / A.P.pass_num, pass = s % A.P.pass_num;
@@ -1138,20 +1034,13 @@ __global__ void __launch_bounds__(kEmitThreads) k_emit(const __grid_constant__ E
       uint8_t *mref = mf + L.refrow_rel, *mread = mf + L.readrow_rel;
       const uint8_t *evbase = A.ev + (A.B.ev_off[s] + (g.segmented ? (uint64_t)tile * PB_SEG_STRIDE : 0ull)) *
                                          (METHOD == PBSIM_METHOD_QSHMM ? 2ull : 1ull);
-      if (!g.slow && BAM) {
-        emit_tile_fast<METHOD, BAM>(evbase, e0, e1, A.G.pk, offset, wlen, minus, ncol, c0.col, c0.ref, c0.read, seq, qual,
-                                    mref, mread, lane, lut_s);
-      } else {
-        RefFetch rf;
-        rf.pk = A.G.pk;
-        rf.ascii = A.G.ascii;
-        rf.offset = offset;
-        rf.wlen = wlen;
-        rf.minus = minus;
-        rf.slow = true;
-        emit_tile_generic<METHOD, BAM>(evbase, e0, e1, rf, minus, ncol, c0.col, c0.ref, c0.read, seq, qual, mref, mread,
-                                       lane, A.philox ? &A.keys : nullptr, (uint32_t)read_id, pass);
-      }
+      RefFetch rf;
+      rf.ascii = A.G.ascii;
+      rf.offset = offset;
+      rf.wlen = wlen;
+      rf.minus = minus;
+      emit_tile_generic<METHOD, BAM>(evbase, e0, e1, rf, minus, ncol, c0.col, c0.ref, c0.read, seq, qual, mref, mread,
+                                     lane, A.philox ? &A.keys : nullptr, (uint32_t)read_id, pass);
     }
     if (A.P.sam) {
       // ip:B:C / pw:B:C arrays: ",9" per read base of this tile (:2324-2331)

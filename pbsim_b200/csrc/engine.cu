@@ -933,6 +933,14 @@ int align_batch(pbsim_engine *e, const EmitArgs &EA, BatchResult *out) {
   return 0;
 }
 
+// K4 per-base rows: the row kernel on the staged tiles, then k_emit on the rest
+template <int METHOD, bool BAM>
+void emit_tiles(pbsim_engine *e, const EmitArgs &EA, uint32_t grid, uint32_t glen_words) {
+  k_emit_rows<METHOD, BAM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, EA.n_tiles, EA.ev, EA.G.pk, glen_words,
+                                                             EA.out_reads, EA.out_maf);
+  k_emit<METHOD, BAM><<<grid, kEmitThreads, 0, e->st>>>(EA);
+}
+
 // K4 record sizes, offsets and text of the reads before the cut, K6 their statistics, and the read-back of their
 // accuracies and lengths
 int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
@@ -1011,26 +1019,18 @@ int emit_batch(pbsim_engine *e, const BatchCtx &c, BatchResult *out) {
     const uint64_t want = (n_tiles + kEmitWarps - 1) / kEmitWarps;
     const uint32_t grid = (uint32_t)std::min<uint64_t>(want, (uint64_t)dev_sms * 8 * 4);
     CK(cudaEventRecord(e->ev_k[2], e->st));
-    // per-tile descriptors (and the tile -> sub-read map), then the row kernel on the plain text tiles and
-    // k_emit on everything else (headers, exceptional / wide tiles, SAM arrays, BAM records)
+    // per-tile descriptors (and the tile -> sub-read map), then the row kernel on the staged tiles and k_emit on
+    // everything else (headers, exceptional / wide tiles, SAM / BAM arrays)
     if (c.qs) k_tile_desc<PBSIM_METHOD_QSHMM><<<nblk(n_tiles, 256), 256, 0, e->st>>>(EA, e->d_tile_sub.as<uint32_t>());
     else k_tile_desc<PBSIM_METHOD_ERRHMM><<<nblk(n_tiles, 256), 256, 0, e->st>>>(EA, e->d_tile_sub.as<uint32_t>());
     e->launches++;
-    if (EA.P.sam == 2u) {  // BAM packs bases with atomic ORs: the records start zeroed
-      CK(cudaMemsetAsync(O.reads.p, 0, (size_t)out->reads_bytes, e->st));
-      if (c.qs) k_emit<PBSIM_METHOD_QSHMM, true><<<grid, kEmitThreads, 0, e->st>>>(EA);
-      else k_emit<PBSIM_METHOD_ERRHMM, true><<<grid, kEmitThreads, 0, e->st>>>(EA);
-    } else {
-      const uint32_t glen_words = (uint32_t)((e->glen + 15) / 16);
-      if (c.qs) {
-        k_emit_rows<PBSIM_METHOD_QSHMM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, n_tiles, EA.ev, c.A.G.pk, glen_words, EA.out_reads, EA.out_maf);
-        k_emit<PBSIM_METHOD_QSHMM, false><<<grid, kEmitThreads, 0, e->st>>>(EA);
-      } else {
-        k_emit_rows<PBSIM_METHOD_ERRHMM><<<grid, kEmitThreads, 0, e->st>>>(EA.desc, n_tiles, EA.ev, c.A.G.pk, glen_words, EA.out_reads, EA.out_maf);
-        k_emit<PBSIM_METHOD_ERRHMM, false><<<grid, kEmitThreads, 0, e->st>>>(EA);
-      }
-      e->launches++;
-    }
+    // BAM packs two bases per byte, and the bytes that two tiles share are ORed in: the records start zeroed
+    const bool bam = EA.P.sam == 2u;
+    if (bam) CK(cudaMemsetAsync(O.reads.p, 0, (size_t)out->reads_bytes, e->st));
+    const uint32_t glen_words = (uint32_t)((e->glen + 15) / 16);
+    if (c.qs) (bam ? emit_tiles<PBSIM_METHOD_QSHMM, true> : emit_tiles<PBSIM_METHOD_QSHMM, false>)(e, EA, grid, glen_words);
+    else (bam ? emit_tiles<PBSIM_METHOD_ERRHMM, true> : emit_tiles<PBSIM_METHOD_ERRHMM, false>)(e, EA, grid, glen_words);
+    e->launches++;
     if (e->align && (rc = align_batch(e, EA, out))) return rc;
     CK(cudaEventRecord(e->ev_k[3], e->st));
     e->launches++;
@@ -1624,10 +1624,9 @@ int pbsim_cuda_create(pbsim_engine **out, int device) {
   // Function attributes belong to the function as loaded on one device, so every engine sets them on its own.
   // k_emit_rows' staging rows need shared memory for 4 CTAs per SM; k_qs_pass1 gets the largest carve-out too.
   CK(cudaFuncSetAttribute(k_qs_pass1, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_QSHMM>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                          cudaSharedmemCarveoutMaxShared));
-  CK(cudaFuncSetAttribute(k_emit_rows<PBSIM_METHOD_ERRHMM>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                          cudaSharedmemCarveoutMaxShared));
+  for (const void *k : {(const void *)k_emit_rows<PBSIM_METHOD_QSHMM, false>, (const void *)k_emit_rows<PBSIM_METHOD_QSHMM, true>,
+                        (const void *)k_emit_rows<PBSIM_METHOD_ERRHMM, false>, (const void *)k_emit_rows<PBSIM_METHOD_ERRHMM, true>})
+    CK(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CK(cudaFuncSetAttribute(k_gz_encode, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGzEncodeSmem));
   pbsim_engine *ne = new pbsim_engine();
   ne->device = device;

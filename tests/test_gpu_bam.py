@@ -66,3 +66,43 @@ def test_bam_of_a_template_run_with_odd_lengths_and_lower_case(eng):
             rows.append("\t".join(f))
         return rows
     assert norm(got) == norm(want)
+
+
+def _genome_with_n_runs(n=160000, seed=3):
+    """random ACGT with an N run of 1..400 bases every 9-23 kb: the tiles next to a run take the generic path, the
+    rest of the record the staged one"""
+    rng = np.random.default_rng(seed)
+    g = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, n)].copy()
+    pos = 4000
+    while pos < n - 1000:
+        g[pos:pos + int(rng.integers(1, 401))] = ord("N")
+        pos += int(rng.integers(9000, 23000))
+    return g.tobytes()
+
+
+@pytest.mark.parametrize("method,model", [("qshmm", "QSHMM-RSII.model"), ("errhmm", "ERRHMM-SEQUEL.model")])
+@pytest.mark.parametrize("segments", [0, 1])
+def test_bam_of_long_reads_across_n_runs_equals_the_sam_text(eng, method, model, segments):
+    """PHILOX mode, reads of several tiles each, so that tiles start and end at odd read positions and staged and
+    generic tiles share a record: the BAM records decode to the SAM text of the same run, the MAF stream is the same"""
+    from tests.golden_util import model_path
+    hm = capi.HostModel(capi.load(), capi.host_params(method, pass_num=2, len_mean=6000.0, len_sd=2500.0),
+                        model_path(model))
+    eng.set_model(hm)
+    genome = _genome_with_n_runs()
+    eng.set_sequence(genome, 1, [0.0] + [1.0] * 10 + [0.0])
+    runs = []
+    eng.set_option("segments", segments)
+    try:
+        for bam in (0, 1):
+            eng.set_option("bam", bam)
+            reads, maf, _, _ = eng.simulate(2 * len(genome), rng_mode=capi.RNG_PHILOX, seed=21)
+            runs.append((reads, maf))
+    finally:
+        eng.set_option("bam", 0)
+        eng.set_option("segments", 1)
+    (sam, maf_sam), (bam, maf_bam) = runs
+    seqs = [ln.split(b"\t")[9] for ln in sam.splitlines()]
+    assert any(b"N" in s and len(s) > 3 * 1024 for s in seqs), "no long record crosses an N run"
+    assert B.records_to_sam(bam) == sam
+    assert maf_bam == maf_sam
