@@ -218,6 +218,11 @@ int pbsim_cuda_set_synthetic_sequence(pbsim_engine *e, int64_t len, int32_t seq_
 int pbsim_cuda_update_hp_del_bias(pbsim_engine *e, const double hp_del_bias[12]);
 /* upper-cased text of the current sequence (tests, benchmarks) */
 int pbsim_cuda_get_sequence_ascii(pbsim_engine *e, char *dst, int64_t cap);
+/* device products of the last set_sequence / set_seqset / set_synthetic_sequence (tests): pk[ceil(len/16)] 2-bit
+ * codes (A=0 C=1 G=2 T=3, base i at bits 2*(i%16) of word i/16), hp4[ceil(len/2)] 4-bit homopolymer lengths (base i
+ * in the low nibble of byte i/2 when i is even), xm[ceil(ceil(len/1024)/32)] exceptional-block bits (block b at bit
+ * b%32 of word b/32).  len must be the current sequence's length. */
+int pbsim_cuda_get_sequence_tables(pbsim_engine *e, uint32_t *pk, uint8_t *hp4, uint32_t *xm, int64_t len);
 /* homopolymer histogram of the current sequence, genome.hpfreq[0..10] plus the aliased [11] */
 int pbsim_cuda_get_hpfreq(pbsim_engine *e, int64_t hpfreq[12]);
 

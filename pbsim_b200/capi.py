@@ -172,7 +172,8 @@ HOST_EXPORTS = ["pbsim_host_sample_filter", "pbsim_host_model_load", "pbsim_host
 ENGINE_EXPORTS = [
     "pbsim_cuda_abi_version", "pbsim_cuda_last_error", "pbsim_cuda_create", "pbsim_cuda_destroy",
     "pbsim_cuda_set_model", "pbsim_cuda_set_sequence", "pbsim_cuda_set_seqset", "pbsim_cuda_set_pool", "pbsim_cuda_set_synthetic_sequence",
-    "pbsim_cuda_update_hp_del_bias", "pbsim_cuda_get_sequence_ascii", "pbsim_cuda_get_hpfreq", "pbsim_cuda_simulate_begin", "pbsim_cuda_next_chunk",
+    "pbsim_cuda_update_hp_del_bias", "pbsim_cuda_get_sequence_ascii", "pbsim_cuda_get_sequence_tables", "pbsim_cuda_get_hpfreq",
+    "pbsim_cuda_simulate_begin", "pbsim_cuda_next_chunk",
     "pbsim_cuda_next_chunk_device", "pbsim_cuda_simulate_end", "pbsim_cuda_stats_device_block",
     "pbsim_cuda_last_chunk_info", "pbsim_cuda_device_timer", "pbsim_cuda_set_option",
     "pbsim_cuda_set_sequence_name",
@@ -215,6 +216,7 @@ def declare_engine(L):
     L.pbsim_cuda_set_synthetic_sequence.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_uint64]
     L.pbsim_cuda_update_hp_del_bias.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
     L.pbsim_cuda_get_sequence_ascii.argtypes = [C.c_void_p, C.c_void_p, C.c_int64]
+    L.pbsim_cuda_get_sequence_tables.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     L.pbsim_cuda_get_hpfreq.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
     L.pbsim_cuda_simulate_begin.argtypes = [C.c_void_p, C.POINTER(Run)]
     L.pbsim_cuda_next_chunk.argtypes = [C.c_void_p, C.POINTER(Chunk)]

@@ -1904,6 +1904,19 @@ int pbsim_cuda_get_sequence_ascii(pbsim_engine *e, char *dst, int64_t cap) {
   return 0;
 }
 
+int pbsim_cuda_get_sequence_tables(pbsim_engine *e, uint32_t *pk, uint8_t *hp4, uint32_t *xm, int64_t len) {
+  if (!e || !pk || !hp4 || !xm || !e->seq_set) return PBSIM_E_INVALID;
+  if (len != e->glen) return fail(e, PBSIM_E_INVALID, "len %lld is not the current sequence's length %lld",
+                                  (long long)len, (long long)e->glen);
+  CK(cudaSetDevice(e->device));
+  const int64_t blocks = (len + (1 << kXmShift) - 1) >> kXmShift;
+  CK(cudaMemcpyAsync(pk, e->d_pk.p, (size_t)((len + 15) / 16) * 4, cudaMemcpyDeviceToHost, e->st));
+  CK(cudaMemcpyAsync(hp4, e->d_hp4.p, (size_t)((len + 1) / 2), cudaMemcpyDeviceToHost, e->st));
+  CK(cudaMemcpyAsync(xm, e->d_xm.p, (size_t)((blocks + 31) / 32) * 4, cudaMemcpyDeviceToHost, e->st));
+  CK(cudaStreamSynchronize(e->st));
+  return 0;
+}
+
 int pbsim_cuda_get_hpfreq(pbsim_engine *e, int64_t hpfreq[12]) {
   if (!e || !e->seq_set) return PBSIM_E_INVALID;
   std::memcpy(hpfreq, e->hpfreq, sizeof e->hpfreq);

@@ -107,9 +107,11 @@ __device__ __forceinline__ uint32_t hp_of(const uint8_t *ascii, int64_t len, int
 
 // One thread per 8 bases (one 32-bit word of hp4), CTAs stride over the sequence.  Runs inside the thread's 8 bytes are
 // measured in registers; only a run that touches the group's first or last byte is followed into the neighbouring
-// text.  The histogram is summed per warp (packed 16-bit counters, REDUX) before it touches shared memory, and every
-// CTA adds its 12 cells to the global histogram once: the one-thread-per-2-bases version spent its time in same-address
-// atomics (1.3 ms per 242 Mbp; this one is bound by the text it reads).
+// text, and only when that byte is not 'N' (N runs of any length are accepted).  A walk capped at 65 536 bases raises
+// *flag: the engine refuses a homopolymer of another letter that long.  The histogram is summed per warp (packed
+// 16-bit counters, REDUX) before it touches shared memory, and every CTA adds its 12 cells to the global histogram
+// once: the one-thread-per-2-bases version spent its time in same-address atomics (1.3 ms per 242 Mbp; this one is
+// bound by the text it reads).
 constexpr int kHpThreads = 256;
 __global__ void __launch_bounds__(kHpThreads) k_hp(const uint8_t *__restrict__ ascii, int64_t len, uint8_t *hp4,
                                                    uint32_t *xm, unsigned long long *hpfreq,
@@ -139,8 +141,11 @@ __global__ void __launch_bounds__(kHpThreads) k_hp(const uint8_t *__restrict__ a
       for (int j = 0; j < 8; ++j) b[j] = (uint8_t)((j < 4 ? v.x : v.y) >> (8 * (j & 3)));
       const int64_t cap = 1 << 16;
       int64_t l = 0, r = 0;
-      while (i0 - l - 1 >= 0 && ascii[i0 - l - 1] == b[0] && l < cap) ++l;
-      while (i0 + 7 + r + 1 < len && ascii[i0 + 7 + r + 1] == b[7] && r < cap) ++r;
+      // left[0] / right[7] only reach bytes equal to b[0] / b[7]; an 'N' gets hp 1 whatever its run: no walk
+      if (b[0] != 'N')
+        while (i0 - l - 1 >= 0 && ascii[i0 - l - 1] == b[0] && l < cap) ++l;
+      if (b[7] != 'N')
+        while (i0 + 7 + r + 1 < len && ascii[i0 + 7 + r + 1] == b[7] && r < cap) ++r;
       if (l >= cap || r >= cap) *flag = 1u;
       uint32_t left[8], right[8];
       left[0] = (uint32_t)l;

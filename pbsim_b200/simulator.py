@@ -114,6 +114,17 @@ class Engine:
     def get_sequence_ascii(self, dst_ptr, cap):
         self._chk(self.L.pbsim_cuda_get_sequence_ascii(self.h, dst_ptr, cap), "get_sequence_ascii")
 
+    def sequence_tables(self):
+        """the ingest products of the current sequence: (pk uint32[ceil(len/16)], hp4 uint8[ceil(len/2)],
+        xm uint32[ceil(ceil(len/1024)/32)])"""
+        n = self.glen
+        pk = np.zeros((n + 15) // 16, dtype=np.uint32)
+        hp4 = np.zeros((n + 1) // 2, dtype=np.uint8)
+        xm = np.zeros(((n + 1023) // 1024 + 31) // 32, dtype=np.uint32)
+        self._chk(self.L.pbsim_cuda_get_sequence_tables(self.h, pk.ctypes.data, hp4.ctypes.data, xm.ctypes.data, n),
+                  "get_sequence_tables")
+        return pk, hp4, xm
+
     def update_bias(self, bias):
         self._chk(self.L.pbsim_cuda_update_hp_del_bias(self.h, (C.c_double * 12)(*bias)), "update_hp_del_bias")
 
