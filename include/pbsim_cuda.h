@@ -146,7 +146,8 @@ typedef struct {
 typedef struct {
   const char *reads;        /* FASTQ (pass_num == 1) or SAM records (no @HD/@RG header)      */
   int64_t reads_bytes;
-  const char *maf;          /* MAF blocks, or with option "align" SAM alignment lines (no header) */
+  const char *maf;          /* MAF blocks, or with option "align" SAM alignment lines (no header), or with
+                             * "align_bam" BAM alignment records (no BAM header; with "deflate", BGZF blocks) */
   int64_t maf_bytes;
   int64_t first_read, n_reads;   /* 1-based id of the first read, number of reads            */
   int64_t bases;                 /* emitted read bases in this chunk, all passes             */
@@ -195,7 +196,8 @@ int pbsim_cuda_set_model(pbsim_engine *e, const pbsim_model *m);
 /* replaces: get_genome_seq's genome.seq / genome.hp (pbsim.cpp:1032-1065): uploads the ASCII
  * sequence, upper-cases, computes homopolymer lengths, packs to 2 bits per base */
 int pbsim_cuda_set_sequence(pbsim_engine *e, const pbsim_sequence *s);
-/* RNAME of the alignment lines of the current WGS sequence (option "align"); required before simulate_begin then.
+/* RNAME of the alignment lines of the current WGS sequence (option "align"); required before simulate_begin then
+ * (not with "align_bam", whose records name the sequence by refID 0).
  * set_sequence and set_synthetic_sequence forget it.  1 to 4096 printable characters, no whitespace. */
 int pbsim_cuda_set_sequence_name(pbsim_engine *e, const char *name);
 /* replaces: the per-sequence ingest of simulate_by_{qshmm,errhmm}_{trans,templ} (upper-casing with the
@@ -259,7 +261,16 @@ int pbsim_cuda_device_timer(pbsim_engine *e, int stop, double *ms);
  * the reads stream, FLAG 0 / 16 (4: no match or substitution column), RNAME (WGS: pbsim_cuda_set_sequence_name; sets:
  * the sequence's id), 1-based POS, MAPQ 60, CIGAR of =, X, I, D in reference order (insertions in front of the first
  * and behind the last = / X column become S, deletions there are dropped), RNEXT * PNEXT 0 TLEN 0, SEQ and QUAL in
- * reference orientation, NM:i; no header lines; not with "bam"; default 0),
+ * reference orientation, NM:i; no header lines; not with "bam" unless "align_bam"; default 0),
+ * "align_bam" (1, needs "align": the second stream holds one BAM alignment record (SAM spec 4.2) per (read, pass)
+ * instead, which decodes to exactly the SAM line "align" writes: refID 0 for WGS (the caller's one @SQ), the sequence's
+ * index in the set for sets, -1 unmapped; pos = POS - 1; MAPQ 60 (unmapped 0); bin = reg2bin(pos, pos + the =, X, D
+ * columns) (unmapped 4680); CIGAR ops = 7, X 8, I 1, D 2, S 4; next refID -1, next pos -1, tlen 0; SEQ as 4-bit codes
+ * high nibble first, the odd pad nibble 0; QUAL values; tag NM of type C, S or I by size.  A record of more than
+ * 65,535 ops holds the two ops <l_seq>S<span>N in its CIGAR field and the real ops in a CG:B:I tag behind NM (SAM spec
+ * 4.2.2).  With "deflate" the records travel as BGZF blocks; the caller writes the BAM header (magic, header text,
+ * n_ref, the references in @SQ order) in front and the BGZF end-of-file block behind.  With "bam" (pass_num > 1)
+ * both streams are BAM.  maf_text_bytes counts the record bytes; default 0),
  * "sample_spec" (--method sample; 1 (default): every copy of a pool entry is first simulated in its own thread at
  * the entry's length and only the copies that follow a shorter read are redone as chains; 0: one thread walks all
  * copies of an entry; results are identical either way; with "segments" the speculative pass of reads of at least

@@ -281,6 +281,7 @@ struct pbsim_engine {
   int deflate = 0;
   int bam = 0;                      // option "bam": multi-pass records are BAM alignment records, not SAM text
   int align = 0;                    // option "align": the second stream holds SAM alignment lines, not MAF blocks
+  int align_bam = 0;                // option "align_bam": with "align", BAM alignment records instead of SAM lines
   std::string seq_name;             // RNAME of WGS alignment lines (pbsim_cuda_set_sequence_name; reset by set_sequence)
   DevBuf d_rname, d_aln_rec, d_aln_maf;
   OutSet gz[2];
@@ -895,7 +896,8 @@ int quota_cut(pbsim_engine *e, BatchCtx &c, int attempt) {
   return 0;
 }
 
-// K5 (option "align"): the MAF blocks pass 2 left in d_aln_maf -> SAM alignment lines in the output set's second stream
+// K5 (option "align"): the MAF blocks pass 2 left in d_aln_maf -> SAM alignment lines (option "align_bam": BAM
+// alignment records) in the output set's second stream
 int align_batch(pbsim_engine *e, const EmitArgs &EA, BatchResult *out) {
   const uint32_t n = EA.n_sub;
   unsigned long long *sam_size = u64_slice(e, kSliceSamSize), *sam_off = u64_slice(e, kSliceSamOff);
@@ -917,7 +919,7 @@ int align_batch(pbsim_engine *e, const EmitArgs &EA, BatchResult *out) {
   A.sam_off = (const uint64_t *)sam_off;
   A.sam = nullptr;
   const uint32_t grid = nblk(n, 8);
-  k_aln_sizes<<<grid, 256, 0, e->st>>>(A, (uint64_t *)sam_size);
+  (e->align_bam ? k_aln_sizes<true> : k_aln_sizes<false>)<<<grid, 256, 0, e->st>>>(A, (uint64_t *)sam_size);
   e->launches++;
   int rc;
   if ((rc = excl_scan(e, sam_size, sam_off, n + 1))) return rc;
@@ -928,7 +930,7 @@ int align_batch(pbsim_engine *e, const EmitArgs &EA, BatchResult *out) {
   pbsim_engine::OutSet &O = e->out[e->cur_set];
   CK(O.maf.ensure((size_t)out->maf_bytes + 256));
   A.sam = O.maf.as<uint8_t>();
-  k_aln_write<<<grid, 256, 0, e->st>>>(A);
+  (e->align_bam ? k_aln_write<true> : k_aln_write<false>)<<<grid, 256, 0, e->st>>>(A);
   e->launches++;
   return 0;
 }
@@ -1303,7 +1305,8 @@ int produce_one(pbsim_engine *e, int set, pbsim_engine::BatchItem *it) {
       // BAM records travel as BGZF blocks (what samtools writes), everything else as plain gzip members
       const bool bgzf = e->bam && e->model.pass_num > 1;
       if ((rc = gz_compress(e, e->out[set].reads.as<uint8_t>(), br.reads_bytes, e->gz[set].reads, &gz_bytes[0], bgzf))) return rc;
-      if ((rc = gz_compress(e, e->out[set].maf.as<uint8_t>(), br.maf_bytes, e->gz[set].maf, &gz_bytes[1]))) return rc;
+      const bool bgzf2 = e->align && e->align_bam;
+      if ((rc = gz_compress(e, e->out[set].maf.as<uint8_t>(), br.maf_bytes, e->gz[set].maf, &gz_bytes[1], bgzf2))) return rc;
       CK(cudaEventRecord(e->ev_gz[1], e->st));
     }
     CK(cudaEventRecord(e->ev1, e->st));
@@ -1929,8 +1932,11 @@ int pbsim_cuda_simulate_begin(pbsim_engine *e, const pbsim_run *run) {
   if (!e->model_set || !e->seq_set) return fail(e, PBSIM_E_INVALID, "set_model and set_sequence must precede simulate_begin");
   if (run->rng_mode == PBSIM_RNG_REPLAY && (!run->replay_draws || !run->replay_starts || run->replay_nsubreads < 1))
     return fail(e, PBSIM_E_INVALID, "replay mode needs the draw log and the subread starts");
-  if (e->align && e->bam) return fail(e, PBSIM_E_INVALID, "options align and bam cannot be combined (alignment lines are SAM text)");
-  if (e->align && e->strategy == PBSIM_STRATEGY_WGS && e->seq_name.empty())
+  if (e->align_bam && !e->align) return fail(e, PBSIM_E_INVALID, "option align_bam needs option align (it sets the encoding of the alignment records)");
+  if (e->align && e->bam && !e->align_bam)
+    return fail(e, PBSIM_E_INVALID, "options align and bam cannot be combined (alignment lines are SAM text)");
+  // BAM records name their sequence by refID 0 (WGS), so only SAM lines need the RNAME
+  if (e->align && !e->align_bam && e->strategy == PBSIM_STRATEGY_WGS && e->seq_name.empty())
     return fail(e, PBSIM_E_INVALID, "option align needs pbsim_cuda_set_sequence_name after set_sequence (the RNAME of the records)");
   // a run abandoned without simulate_end: its producer thread must be gone before any run state changes
   stop_producer(e);
@@ -2132,6 +2138,11 @@ int pbsim_cuda_set_option(pbsim_engine *e, const char *name, int64_t value) {
   if (!strcmp(name, "align")) {
     if (e->running) return fail(e, PBSIM_E_INVALID, "align cannot change during a run");
     e->align = value != 0;
+    return 0;
+  }
+  if (!strcmp(name, "align_bam")) {
+    if (e->running) return fail(e, PBSIM_E_INVALID, "align_bam cannot change during a run");
+    e->align_bam = value != 0;
     return 0;
   }
   if (!strcmp(name, "deflate")) {

@@ -73,6 +73,7 @@ struct Options {
                              // (n - 1) % world == rank (their output files are independent of everything else)
   std::string gzip = "gpu";  // who writes the gzip members: the GPU (gz_kernels.cuh) or zlib threads on the host
   std::string align = "maf"; // the second file: MAF blocks (.maf.gz) or SAM alignment lines (.aln.sam.gz)
+  std::string align_encoding = "text";  // --align sam: SAM text (.aln.sam.gz) or BAM records (.aln.bam)
 };
 
 std::thread *g_background = nullptr;  // a thread that must have ended before the process exits (CUDA start-up)
@@ -378,7 +379,7 @@ void stream_to(GzipWriter &w, const char *p, int64_t n, bool raw = false) {
   for (int64_t o = 0; o < n; o += blk) w.submit(p + o, (size_t)std::min(blk, n - o), raw);
 }
 
-// one BGZF block (SAM spec 4.1) holding `data` (at most 64 KiB): the BAM file header goes through here, the
+// one BGZF block (SAM spec 4.1) holding `data` (at most 64 KiB): the BAM file headers go through here, the
 // alignment records arrive from the GPU as BGZF blocks already
 std::string bgzf_block(const std::string &data) {
   z_stream zs;
@@ -772,7 +773,9 @@ void print_help() {
           "                       output is <prefix>_NNNN.bam) | host: zlib threads (multi-pass: .sam.gz).\n"
           "  --align              maf (default): alignments as MAF, <prefix>_NNNN.maf.gz | sam: each read's true\n"
           "                       alignment as a SAM line with a CIGAR, <prefix>_NNNN.aln.sam.gz (with --pass-num > 1\n"
-          "                       it needs --gzip host).\n\n"
+          "                       it needs --gzip host).\n"
+          "  --align-encoding     text (default) | bam: with --align sam, BAM records in <prefix>_NNNN.aln.bam\n"
+          "                       (needs --gzip gpu; allows --pass-num > 1).\n\n"
           " [options for transcriptome / template sequencing]\n\n"
           "  --strategy           trans | templ\n"
           "  --transcript         transcript table: id, plus count, minus count, sequence (tab separated).\n"
@@ -817,7 +820,7 @@ int main(int argc, char **argv) {
       {"gpu", 1, nullptr, 0},        {"rng", 1, nullptr, 0},            {"replay-draws", 1, nullptr, 0},
       {"replay-marks", 1, nullptr, 0}, {"threads", 1, nullptr, 0},      {"gzip", 1, nullptr, 0},
       {"rank", 1, nullptr, 0},       {"world", 1, nullptr, 0},          {"align", 1, nullptr, 0},
-      {nullptr, 0, nullptr, 0}};
+      {"align-encoding", 1, nullptr, 0}, {nullptr, 0, nullptr, 0}};
   int opt, idx = 0;
   while ((opt = getopt_long(argc, argv, "", long_options, &idx)) != -1) {
     if (opt != 0) exit(-1);
@@ -918,6 +921,10 @@ int main(int argc, char **argv) {
         if (!strcmp(a, "maf") || !strcmp(a, "sam")) o.align = a;
         else die("ERROR (align: %s): Acceptable value: maf, sam.\n", a);
         break;
+      case 32:
+        if (!strcmp(a, "text") || !strcmp(a, "bam")) o.align_encoding = a;
+        else die("ERROR (align-encoding: %s): Acceptable value: text, bam.\n", a);
+        break;
       default: break;
     }
   }
@@ -933,6 +940,9 @@ int main(int argc, char **argv) {
   if (o.strategy == "templ" && !o.set_flg[21]) die("ERROR: for --strategy templ, --template must be set.\n");
   if (o.method == "qshmm" && !o.set_flg[15]) die("ERROR: for --method qshmm, --qshmm must be set.\n");
   if (o.method == "errhmm" && !o.set_flg[16]) die("ERROR: for --method errhmm, --errhmm must be set.\n");
+  if (o.align_encoding == "bam" && o.align != "sam") die("ERROR: --align-encoding bam needs --align sam.\n");
+  if (o.align_encoding == "bam" && o.gzip != "gpu")
+    die("ERROR: --align-encoding bam needs --gzip gpu (the host writer produces gzip members, not BGZF blocks).\n");
   // sample, sample-profile-id (:1565-1616): --sample alone filters the FASTQ, with a profile id the filtered reads are
   // stored (sample_profile_<id>.fastq / .stats), the id alone reuses a stored profile
   const bool sample = o.method == "sample";
@@ -1182,15 +1192,40 @@ int main(int argc, char **argv) {
   const bool bam = o.pass_num > 1 && o.gzip == "gpu";
   if (pbsim_cuda_set_option(eng, "bam", bam ? 1 : 0) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
   const bool align = o.align == "sam";
-  if (align && bam) die("ERROR: --align sam with --pass-num > 1 needs --gzip host (BAM reads and SAM alignment lines are not written together).\n");
+  const bool align_bam = align && o.align_encoding == "bam";
+  if (align && bam && !align_bam)
+    die("ERROR: --align sam with --pass-num > 1 needs --gzip host (BAM reads and SAM alignment lines are not written together).\n");
   if (pbsim_cuda_set_option(eng, "align", align ? 1 : 0) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
-  // sq: the @SQ lines of the alignment file (--align sam)
-  auto simulate_to_files = [&](const std::string &stem, const std::string &pu, int64_t len_quota, const std::string &sq) {
+  if (pbsim_cuda_set_option(eng, "align_bam", align_bam ? 1 : 0) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
+  // sq: the @SQ lines of the alignment file (--align sam), (name, length) each
+  auto simulate_to_files = [&](const std::string &stem, const std::string &pu, int64_t len_quota,
+                               const std::vector<std::pair<std::string, int64_t>> &sq) {
     GzipWriter reads_out((stem + (o.pass_num == 1 ? ".fq.gz" : (bam ? ".bam" : ".sam.gz"))).c_str(), std::max(1, threads / 2));
-    GzipWriter maf_out((stem + (align ? ".aln.sam.gz" : ".maf.gz")).c_str(), std::max(1, threads / 2));
+    GzipWriter maf_out((stem + (align_bam ? ".aln.bam" : (align ? ".aln.sam.gz" : ".maf.gz"))).c_str(), std::max(1, threads / 2));
     if (align) {
-      const std::string h = "@HD\tVN:1.6\tSO:unknown\n" + sq + "@PG\tID:pbsim\tPN:pbsim\n";
-      maf_out.submit(h.data(), h.size());
+      std::string h = "@HD\tVN:1.6\tSO:unknown\n";
+      for (const auto &r : sq) h += "@SQ\tSN:" + r.first + "\tLN:" + std::to_string(r.second) + "\n";
+      h += "@PG\tID:pbsim\tPN:pbsim\n";
+      if (align_bam) {
+        // BAM file header (SAM spec 4.2): magic, the header text, then n_ref and every reference in @SQ order, in as
+        // many BGZF blocks as it takes (a transcript table of a few thousand ids outgrows one)
+        std::string b("BAM\1", 4);
+        auto put32 = [&b](uint32_t v) { b.append(reinterpret_cast<const char *>(&v), 4); };
+        put32((uint32_t)h.size());
+        b += h;
+        put32((uint32_t)sq.size());
+        for (const auto &r : sq) {
+          put32((uint32_t)r.first.size() + 1u);
+          b.append(r.first.c_str(), r.first.size() + 1);
+          put32((uint32_t)r.second);
+        }
+        for (size_t at = 0; at < b.size(); at += 0xff00) {  // htslib's block size: BSIZE fits 16 bits
+          const std::string blk = bgzf_block(b.substr(at, 0xff00));
+          maf_out.submit(blk.data(), blk.size(), true);
+        }
+      } else {
+        maf_out.submit(h.data(), h.size());
+      }
     }
     if (o.pass_num > 1) {  // SAM header (:721-722, :781-782)
       char hdr[1024];
@@ -1252,11 +1287,11 @@ int main(int argc, char **argv) {
     }
     pbsim_stats st;
     if (pbsim_cuda_simulate_end(eng, &st, nullptr, 0, nullptr) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
-    if (bam) {  // BGZF end-of-file marker (SAM spec 4.1.2)
-      static const unsigned char eof[28] = {0x1f, 0x8b, 0x08, 0x04, 0, 0, 0, 0, 0, 0xff, 0x06, 0, 0x42, 0x43,
-                                            0x02, 0, 0x1b, 0, 0x03, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-      reads_out.submit(reinterpret_cast<const char *>(eof), sizeof eof, true);
-    }
+    // BGZF end-of-file marker (SAM spec 4.1.2)
+    static const unsigned char eof[28] = {0x1f, 0x8b, 0x08, 0x04, 0, 0, 0, 0, 0, 0xff, 0x06, 0, 0x42, 0x43,
+                                          0x02, 0, 0x1b, 0, 0x03, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (bam) reads_out.submit(reinterpret_cast<const char *>(eof), sizeof eof, true);
+    if (align_bam) maf_out.submit(reinterpret_cast<const char *>(eof), sizeof eof, true);
     reads_out.close();
     maf_out.close();
     replay_pos += (size_t)st.res_pass_num;
@@ -1315,9 +1350,8 @@ int main(int argc, char **argv) {
       pbsim_host_hp_del_bias(o.hp_del_bias, f, ss.hp_del_bias);
       if (pbsim_cuda_set_seqset(eng, &ss) != 0) die("ERROR: %s\n", pbsim_cuda_last_error(eng));
     }
-    std::string sq;
-    for (size_t t = 0; align && t < S.ids.size(); ++t)
-      sq += "@SQ\tSN:" + S.ids[t] + "\tLN:" + std::to_string(S.start[t + 1] - S.start[t]) + "\n";
+    std::vector<std::pair<std::string, int64_t>> sq;
+    for (size_t t = 0; align && t < S.ids.size(); ++t) sq.emplace_back(S.ids[t], (int64_t)(S.start[t + 1] - S.start[t]));
     const pbsim_stats st = simulate_to_files(o.prefix, o.id_prefix, 0, sq);
     fprintf(stderr, ":::: Simulation stats ::::\n\n");
     fprintf(stderr, "read num. : %ld\n", (long)st.res_num);
@@ -1369,7 +1403,8 @@ int main(int argc, char **argv) {
     char stem[4096], pu[512];
     snprintf(stem, sizeof stem, "%s_%04zu", o.prefix.c_str(), n);
     snprintf(pu, sizeof pu, "%s%zu", o.id_prefix.c_str(), n);
-    const std::string sq = align ? "@SQ\tSN:" + seq_name(n) + "\tLN:" + std::to_string(glen) + "\n" : "";
+    std::vector<std::pair<std::string, int64_t>> sq;
+    if (align) sq.emplace_back(seq_name(n), (int64_t)glen);
     const pbsim_stats st = simulate_to_files(stem, pu, (int64_t)(o.depth * glen), sq);  // sim.len_quota (:705)
     // print_simulation_stats (:5541-5564)
     fprintf(stderr, ":::: Simulation stats (ref.%zu) ::::\n\n", n);
